@@ -34,6 +34,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -43,6 +44,7 @@ UNIT = "steps/s"
 W_ALG = 7             # fp32 lane-ops per useful step in the reference's unfused form (SURVEY 8d)
 BYTES_PER_TRIAL = 348  # 340 B of z in + 8 B of x out
 P = 80
+DUMP_ROWS = 1 << 21    # --dump-outputs: 16 MB of the 800 MB x of a 1e8-trial step
 
 
 def parse():
@@ -66,6 +68,10 @@ def parse():
                     help="configs[4]: SBC datasets per GPU (1000 on 8 GPUs); 0 skips it")
     ap.add_argument("--train-set-trials", type=int, default=int(os.environ.get("DDM_BENCH_TRAINSET_TRIALS", 10_000_000)),
                     help="end-to-end simulate_training_set_with_conditions leg (N=1 only); 0 skips it")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write x of the last timed step to DIR/x.npy (float32, (rows, 2)) so that two builds can be "
+                         f"compared: every row when there are at most {DUMP_ROWS}, else {DUMP_ROWS} rows drawn without "
+                         "replacement by numpy default_rng(0), in ascending row order")
     return ap.parse_args()
 
 
@@ -224,6 +230,17 @@ def build_workload(n: int, rank: int, device):
     pulses_from_state(state, inc, rank * n, n, P, 0.75, out=z[:, 5:])
     return z
 
+
+def dump_outputs(out_dir: str, x) -> None:
+    """x (device, (n, 2) float32) as out_dir/x.npy: all rows, or DUMP_ROWS of them sampled with a fixed seed."""
+    import numpy as np
+    import torch
+    n = x.shape[0]
+    if n > DUMP_ROWS:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+        x = x[torch.from_numpy(rows).to(x.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "x.npy"), x.cpu().numpy().astype(np.float32))
 
 
 # ------------------------------------------------------------------- MNLE potential (cfg-4) ---
@@ -798,6 +815,8 @@ def run_native(args):
     clock_info = clocks.stop()
     elapsed_ms = t_start.elapsed_time(t_end)
     kernel_ms = [a.elapsed_time(b) for a, b in kernel_events]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, x_all if x_all is not None else x)
 
     # ---- N > 1: the gathered x of the last timed step equals a single-rank recomputation -------------
     # Every rank takes 65 536 rows of the NEXT rank's z (all-gathered), simulates them alone with that
