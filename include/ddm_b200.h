@@ -244,8 +244,10 @@ int ddm_pcg64_advance(uint64_t *state_hi, uint64_t *state_lo, uint64_t inc_hi, u
  */
 size_t mnle_packed_floats(int n_choices);
 
-/* Copies the packed parameters to the current device; *handle_out is an opaque read-only
- * handle owned by the caller (mnle_destroy).  One handle per (process, device). */
+/* Copies the packed parameters to the current device and builds the tensor-core operand pack
+ * from them there: one kernel on the legacy default stream, waited for before the call returns.
+ * *handle_out is an opaque read-only handle owned by the caller (mnle_destroy).  One handle per
+ * (process, device). */
 int mnle_create(const float *packed_host, size_t n_floats, int n_choices, void **handle_out);
 int mnle_destroy(void *handle);
 

@@ -92,13 +92,12 @@ struct Handle {
     int device;
     Layout layout;
     float *params;   // device copy of the packed buffer
-    void *tc_pack;   // device copy of the tensor-core operand pack (bf16 hi/lo tiles), or null
-    size_t tc_pack_bytes;
+    void *tc_pack;   // tensor-core operand pack (bf16 hi/lo tiles) built on the device from params, or null
     TcPlan tc_plan;       // potential mode: rows = (trial, chain), first layers hoisted per trial
     TcPlan tc_rows_plan;  // rows mode: arbitrary (R, 85) conditions, first layers on the tensor cores
     float mu_y, sigma_y;
 };
-int build_tc_pack(Handle *H, const float *packed_host);  // mnle_tc.cu
+int tc_handle_pack(Handle *H);  // mnle_tc.cu: allocates and writes tc_pack, sets both plans
 
 // Training forward on the tensor cores (mnle_tc.cu): the rows-mode kernel over the minibatch with the
 // operand pack rebuilt on the device from the current parameters, keeping what the backward pass needs.

@@ -157,7 +157,6 @@ DDM_API int mnle_create(const float *packed_host, size_t n_floats, int n_choices
     H->magic = kMagic;
     H->layout = L;
     H->tc_pack = nullptr;
-    H->tc_pack_bytes = 0;
     H->params = nullptr;
     H->mu_y = packed_host[L.mu_y];
     H->sigma_y = sigma;
@@ -168,7 +167,7 @@ DDM_API int mnle_create(const float *packed_host, size_t n_floats, int n_choices
         delete H;
         return ddm::cuda_fail(e, "mnle_create");
     }
-    const int rc = build_tc_pack(H, packed_host);
+    const int rc = tc_handle_pack(H);
     if (rc != DDM_OK) {
         cudaFree(H->params);
         if (H->tc_pack) cudaFree(H->tc_pack);

@@ -7,10 +7,6 @@
 // TMEM): 16 mantissa bits per operand at 3/2 of the cost of a tf32 product.
 //
 // This file: the operand layout / descriptor self-test (mnle_tc_selftest) and the fused kernel.
-#include <string.h>
-
-#include <vector>
-
 #include "mnle_common.cuh"
 #include "tc_ptx.cuh"
 
@@ -138,142 +134,6 @@ __global__ void __launch_bounds__(128) tc_selftest_kernel(const float *__restric
     if (warp == 0) tmem_dealloc<256>(tmem);
 }
 
-
-// ------------------------------------------------------------- operand pack (host side) ---
-// Round-to-nearest-even fp32 -> bf16, the same rounding as __float2bfloat16_rn.
-static inline uint16_t host_bf16(float x)
-{
-    uint32_t u;
-    memcpy(&u, &x, 4);
-    if ((u & 0x7F800000u) == 0x7F800000u) return (uint16_t)(u >> 16);  // inf / nan
-    u += 0x7FFFu + ((u >> 16) & 1u);
-    return (uint16_t)(u >> 16);
-}
-static inline float host_bf16_to_f(uint16_t h)
-{
-    const uint32_t u = (uint32_t)h << 16;
-    float f;
-    memcpy(&f, &u, 4);
-    return f;
-}
-// x = t[0] + t[1] + t[2] + O(2^-25 |x|)
-static inline void host_split3(float x, uint16_t (&t)[3])
-{
-    float r = x;
-    for (int i = 0; i < 3; ++i) {
-        t[i] = host_bf16(r);
-        r -= host_bf16_to_f(t[i]);
-    }
-}
-
-// K = 128 weight image of one bf16 term (0 = hi, 1 = lo) of W[n_valid][128], padded to N rows.
-static void pack_image_k128(std::vector<unsigned char> &blob, const float *W, int n_valid, int N, int term)
-{
-    const size_t base = blob.size();
-    blob.resize(base + (size_t)N * 256, 0);
-    for (int n = 0; n < n_valid; ++n)
-        for (int k = 0; k < kHidden; ++k) {
-            uint16_t t[3];
-            host_split3(W[(size_t)n * kHidden + k], t);
-            memcpy(&blob[base + tile_offset(N, n, k)], &t[term], 2);
-        }
-}
-static void pack_bias(std::vector<unsigned char> &blob, const float *b, int n_valid, int N)
-{
-    const size_t base = blob.size();
-    blob.resize(base + (size_t)N * 4, 0);
-    memcpy(&blob[base], b, (size_t)n_valid * 4);
-}
-// theta stage: image [128][32]; k = term * 5 + i pairs with the A image built by the kernel.
-//   A terms: t1 t1 t2 t1 t2 t3      B terms: w1 w2 w1 w3 w2 w1     (all products of order <= 4)
-static void pack_image_theta(std::vector<unsigned char> &blob, const float *W1, int ldw)
-{
-    static const int wterm[6] = {0, 1, 0, 2, 1, 0};
-    const size_t base = blob.size();
-    blob.resize(base + (size_t)kHidden * 64, 0);
-    for (int n = 0; n < kHidden; ++n)
-        for (int i = 0; i < 5; ++i) {
-            uint16_t t[3];
-            host_split3(W1[(size_t)n * ldw + i], t);
-            for (int term = 0; term < 6; ++term)
-                memcpy(&blob[base + tile_offset(kHidden, n, term * 5 + i)], &t[wterm[term]], 2);
-        }
-}
-
-int build_tc_pack(Handle *H, const float *packed_host)
-{
-    const Layout &L = H->layout;
-    std::vector<unsigned char> blob;
-    TcPlan &P = H->tc_plan;
-    int s = 0;
-    auto begin = [&](int n, int kind, int epi, int net) {
-        P.st[s].off = (uint32_t)blob.size();
-        P.st[s].n = (uint16_t)n;
-        P.st[s].kind = (uint8_t)kind;
-        P.st[s].epi = (uint8_t)epi;
-        P.st[s].net = (uint16_t)net;
-    };
-    auto end = [&](bool bias_in_blob) {
-        P.st[s].bytes = (uint32_t)blob.size() - P.st[s].off;
-        P.st[s].bias_off = bias_in_blob ? P.st[s].bytes - (uint32_t)P.st[s].n * 4u : P.st[s].bytes;
-        ++s;
-    };
-    auto dense = [&](size_t W, size_t b, int n_valid, int N, int epi, int net) {
-        begin(N, kStageK128, epi, net);
-        pack_image_k128(blob, packed_host + W, n_valid, N, 0);
-        pack_image_k128(blob, packed_host + W, n_valid, N, 1);
-        pack_bias(blob, packed_host + b, n_valid, N);
-        end(true);
-    };
-    // categorical net
-    begin(kHidden, kStageTheta, kEpiSigmoid, 0);
-    pack_image_theta(blob, packed_host + L.cat_W0, kCond);
-    end(false);
-    dense(L.cat_W1, L.cat_b1, kHidden, kHidden, kEpiSigmoid, 0);
-    dense(L.cat_W2, L.cat_b2, kHidden, kHidden, kEpiSigmoid, 0);
-    dense(L.cat_Wo, L.cat_bo, L.n_choices, 16, kEpiCategorical, 0);
-    for (int k = 0; k < kTransforms; ++k) {
-        begin(kHidden, kStageTheta, kEpiRelu, 1 + k);
-        pack_image_theta(blob, packed_host + L.fl_W1[k], kCtx);
-        end(false);
-        dense(L.fl_W2[k], L.fl_b2[k], kHidden, kHidden, kEpiRelu, 1 + k);
-        dense(L.fl_W3[k], L.fl_b3[k], kSplineOut, kSplineN, kEpiSpline, 1 + k);
-    }
-    if (s != kTcStages) {
-        ddm::set_error("build_tc_pack: %d stages, expected %d", s, kTcStages);
-        return DDM_ERR_STATE;
-    }
-    // rows mode: the same plan with every theta stage replaced by the whole first layer (K = 96)
-    TcPlan &R = H->tc_rows_plan;
-    R = P;
-    for (int i = 0; i < kTcStages; ++i) {
-        if (P.st[i].kind != kStageTheta) continue;
-        const int net = P.st[i].net;
-        const float *W = packed_host + (net == 0 ? L.cat_W0 : L.fl_W1[net - 1]);
-        const float *b = packed_host + (net == 0 ? L.cat_b0 : L.fl_b1[net - 1]);
-        const int K = net == 0 ? kCond : kCtx;
-        TcStage &st = R.st[i];
-        st.off = (uint32_t)blob.size();
-        st.kind = kStageInput;
-        for (int term = 0; term < 2; ++term) {
-            const size_t base = blob.size();
-            blob.resize(base + (size_t)kHidden * kInputK * 2, 0);
-            for (int n = 0; n < kHidden; ++n)
-                for (int k = 0; k < K; ++k) {
-                    uint16_t t[3];
-                    host_split3(W[(size_t)n * K + k], t);
-                    memcpy(&blob[base + tile_offset(kHidden, n, k)], &t[term], 2);
-                }
-        }
-        pack_bias(blob, b, kHidden, kHidden);
-        st.bytes = (uint32_t)blob.size() - st.off;
-        st.bias_off = st.bytes - (uint32_t)kHidden * 4u;
-    }
-    DDM_CUDA_TRY(cudaMalloc(&H->tc_pack, blob.size()));
-    DDM_CUDA_TRY(cudaMemcpy(H->tc_pack, blob.data(), blob.size(), cudaMemcpyHostToDevice));
-    H->tc_pack_bytes = blob.size();
-    return DDM_OK;
-}
 
 // ---------------------------------------------------------------- per-trial first layer ---
 // hoist[t][net][j] = b1[j] + sum_i W1[j][5 + i] * pulses[t][i] (+ W1[j][85] * choice[t] for the
@@ -852,7 +712,7 @@ __global__ void __launch_bounds__(kTcThreads, 1)
                 *reinterpret_cast<uint4 *>(img_hi + off) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
                 *reinterpret_cast<uint4 *>(img_lo + off) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
             }
-        } else {   // A image of the theta stage: k = term * 5 + i, terms t1 t1 t2 t1 t2 t3 (pairs with pack_image_theta)
+        } else {   // A image of the theta stage: k = term * 5 + i, terms t1 t1 t2 t1 t2 t3 (pairs with tc_pack_job's theta image)
             unsigned char *a_th = smem + kSmemATh + (uint32_t)X * kAThBytes;
             uint16_t tt[5][3];
 #pragma unroll
@@ -1041,35 +901,52 @@ __global__ void __launch_bounds__(kTcThreads, 1)
     if (warp == kTcEpiWarps) tmem_dealloc<512>(tmem);
 }
 
-// ------------------------------------------------------------ training forward (row f4) ---
-// The parameters change every optimisation step, so the rows-mode operand pack (bf16 hi / lo images in
-// the UMMA shared-memory layout + fp32 biases, same format as build_tc_pack's) is rebuilt on the device.
+// ------------------------------------------------------------------------ operand packs ---
+// Every operand pack is written on the device from the packed fp32 parameters (tc_prep_kernel), one pack job
+// per stage blob: the handle's pack once, when mnle_create has copied the parameters, and the training pack
+// every optimisation step, because the parameters change.
+enum PackKind : uint16_t {
+    kPackDense = 0,       // image row = row of W, k = column of W: hi image, lo image, bias
+    kPackTransposed = 1,  // image row = column of W, k = row of W: hi image, lo image (backward-data stages)
+    kPackTheta = 2,       // theta image of W's first five columns (tc_pack_job): one image, no bias
+};
 struct PackJob {
     uint32_t w_off, b_off;      // weight / bias position in the packed parameters (floats)
     uint32_t dst, img_bytes;    // blob position in the pack, bytes of one image (hi; lo follows)
     uint16_t n_valid, k_valid;  // W is [n_valid][k_valid] row-major
-    uint16_t n_img, transpose;  // rows of the image (UMMA N); transpose: image row = column of W, k = row of W
+    uint16_t n_img, kind;       // rows of the image (UMMA N); PackKind
 };
 constexpr int kTrainStages = kTcStages + 3 + 2 * kTransforms;  // forward stages + backward-data stages
 struct PackJobs {
-    PackJob j[kTrainStages];
+    PackJob j[kTrainStages];  // (the training pack has the most jobs)
+    int n;
 };
 
 constexpr int kPackSplit = 8;  // CTAs per pack job
 
-// One launch prepares everything the step's tensor-core kernels read: CTAs [0, kTrainStages * kPackSplit)
-// rebuild the operand pack from the current parameters -- every byte of it, padding rows / columns and
-// padding biases included, so the caller's workspace needs no clearing --, the others build the context
-// images of one row tile each (tc_ctx_tile below).
+// One launch prepares everything the tensor-core kernels read: CTAs [0, jobs.n * kPackSplit) write the
+// operand pack from the current parameters -- every byte of it, padding rows / columns and padding biases
+// included, so the caller's workspace needs no clearing --, the others build the context images of one row
+// tile each (tc_ctx_tile below).
 __device__ __forceinline__ void tc_pack_job(const float *__restrict__ params, const PackJob &J, int part,
                                             unsigned char *__restrict__ pack)
 {
     const int n_img = J.n_img, k_img = (int)(J.img_bytes / (2u * J.n_img));
     const int total = n_img * k_img;
     for (int idx = part * blockDim.x + threadIdx.x; idx < total; idx += kPackSplit * blockDim.x) {
+        if (J.kind == kPackTheta) {
+            // [n_img][32]: k = term * 5 + i holds term {0, 1, 0, 2, 1, 0}[term] of the three-term split of W[r][i],
+            // paired with the A terms t1 t1 t2 t1 t2 t3 mnle_tc_kernel builds (all products of order <= 4); k = 30, 31: 0
+            const int r = idx / k_img, k = idx - r * k_img, term = k / 5;
+            uint16_t t[3] = {0, 0, 0};
+            if (k < 30) split3_bf16(params[J.w_off + r * J.k_valid + (k - 5 * term)], t);
+            *reinterpret_cast<uint16_t *>(pack + J.dst + tile_offset(n_img, r, k)) =
+                term == 3 ? t[2] : (term == 1 || term == 4) ? t[1] : t[0];
+            continue;
+        }
         int r, k;  // image row, k; consecutive threads read consecutive parameters
         float v = 0.f;
-        if (!J.transpose) {
+        if (J.kind == kPackDense) {
             r = idx / k_img;
             k = idx - r * k_img;
             if (r < J.n_valid && k < J.k_valid) v = params[J.w_off + r * J.k_valid + k];
@@ -1084,17 +961,21 @@ __device__ __forceinline__ void tc_pack_job(const float *__restrict__ params, co
         *reinterpret_cast<uint16_t *>(pack + off) = hi;
         *reinterpret_cast<uint16_t *>(pack + off + J.img_bytes) = lo;
     }
-    if (part == 0 && !J.transpose)  // (the backward-data stages have no bias)
+    if (part == 0 && J.kind == kPackDense)
         for (int n = threadIdx.x; n < n_img; n += blockDim.x)
             reinterpret_cast<float *>(pack + J.dst + 2 * J.img_bytes)[n] = n < J.n_valid ? params[J.b_off + n] : 0.f;
 }
 
-// stage plans of the training forward and backward-data passes over one pack that holds exactly their
-// stages, in order (forward stages first)
-static size_t train_plan(const Layout &L, TcPlan *plan, TcPlan *bplan, PackJobs *jobs)
+// Stage plans and pack jobs of the two operand packs (null outputs are skipped); returns the pack's bytes.
+// Both packs start with the forward stages, in `plan` (the rows-mode plan): cat (first layer, W1, W2, Wo),
+// then flow 0..9 (first layer, W2, W3), every first layer a K = 96 stage.  The training pack (theta = false)
+// continues with the backward-data stages, in `tail` in the order of the backward pass; the handle's pack
+// (theta = true) with one theta stage per net, net i's in tail->st[i].
+static size_t pack_plan(const Layout &L, bool theta, TcPlan *plan, TcPlan *tail, PackJobs *jobs)
 {
     size_t bytes = 0;
-    int s = 0, nj = 0;
+    int s = 0;
+    if (jobs) jobs->n = 0;
     auto stage = [&](size_t W, size_t b, int n_valid, int k_valid, int n_img, int k_img, int kind, int epi, int net, int slot) {
         const uint32_t img = (uint32_t)n_img * (uint32_t)k_img * 2u;
         if (plan) {
@@ -1109,11 +990,10 @@ static size_t train_plan(const Layout &L, TcPlan *plan, TcPlan *bplan, PackJobs 
             st.pad = (uint16_t)slot;
         }
         if (jobs)
-            jobs->j[nj] = PackJob{(uint32_t)W, (uint32_t)b, (uint32_t)bytes, img, (uint16_t)n_valid, (uint16_t)k_valid,
-                                  (uint16_t)n_img, 0};
+            jobs->j[jobs->n++] = PackJob{(uint32_t)W, (uint32_t)b, (uint32_t)bytes, img, (uint16_t)n_valid,
+                                         (uint16_t)k_valid, (uint16_t)n_img, kPackDense};
         bytes += 2u * img + (uint32_t)n_img * 4u;
         ++s;
-        ++nj;
     };
     stage(L.cat_W0, L.cat_b0, kHidden, kCond, kHidden, kInputK, kStageInput, kEpiSigmoid, 0, 1);
     stage(L.cat_W1, L.cat_b1, kHidden, kHidden, kHidden, kHidden, kStageK128, kEpiSigmoid, 0, 2);
@@ -1124,12 +1004,29 @@ static size_t train_plan(const Layout &L, TcPlan *plan, TcPlan *bplan, PackJobs 
         stage(L.fl_W2[k], L.fl_b2[k], kHidden, kHidden, kHidden, kHidden, kStageK128, kEpiRelu, 1 + k, 2);
         stage(L.fl_W3[k], L.fl_b3[k], kSplineOut, kHidden, kSplineN, kHidden, kStageK128, kEpiSpline, 1 + k, 0);
     }
+    if (theta) {
+        // theta stage: the image alone; its bias is the net's per-trial first-layer sum (mnle_hoist_kernel),
+        // which the potential kernel stages right behind the image
+        auto tstage = [&](size_t W, int ldw, int epi, int net) {
+            const uint32_t img = (uint32_t)kHidden * 32u * 2u;
+            if (tail)
+                tail->st[net] = TcStage{(uint32_t)bytes, img, img, (uint16_t)kHidden, (uint8_t)kStageTheta, (uint8_t)epi,
+                                        (uint16_t)net, 0};
+            if (jobs)
+                jobs->j[jobs->n++] = PackJob{(uint32_t)W, 0u, (uint32_t)bytes, img, (uint16_t)kHidden, (uint16_t)ldw,
+                                             (uint16_t)kHidden, kPackTheta};
+            bytes += img;
+        };
+        tstage(L.cat_W0, kCond, kEpiSigmoid, 0);
+        for (int k = 0; k < kTransforms; ++k) tstage(L.fl_W1[k], kCtx, kEpiRelu, 1 + k);
+        return bytes;
+    }
     // backward-data: out[row][in] = sum_out g[row][out] W[out][in]  ->  B image = W transposed ([in][out], K = out)
     int bs = 0;
     auto bstage = [&](size_t W, int n_out, int n_in, int k_img, int kind, int epi, int net, int mask_slot) {
         const uint32_t img = (uint32_t)kHidden * (uint32_t)k_img * 2u;  // n_in = 128 rows everywhere
-        if (bplan) {
-            TcStage &st = bplan->st[bs];
+        if (tail) {
+            TcStage &st = tail->st[bs];
             st.off = (uint32_t)bytes;
             st.bytes = 2u * img;
             st.bias_off = 2u * img;
@@ -1140,10 +1037,10 @@ static size_t train_plan(const Layout &L, TcPlan *plan, TcPlan *bplan, PackJobs 
             st.pad = (uint16_t)((mask_slot + 1) | ((k_img / 16) << 8));
         }
         if (jobs)
-            jobs->j[nj] = PackJob{(uint32_t)W, 0u, (uint32_t)bytes, img, (uint16_t)n_out, (uint16_t)n_in, (uint16_t)kHidden, 1};
+            jobs->j[jobs->n++] = PackJob{(uint32_t)W, 0u, (uint32_t)bytes, img, (uint16_t)n_out, (uint16_t)n_in,
+                                         (uint16_t)kHidden, kPackTransposed};
         bytes += 2u * img;
         ++bs;
-        ++nj;
     };
     bstage(L.cat_Wo, L.n_choices, kHidden, 16, kStageInput, kEpiSigmoid, 0, 2);
     bstage(L.cat_W2, kHidden, kHidden, kHidden, kStageK128, kEpiSigmoid, 0, 1);
@@ -1197,14 +1094,32 @@ __global__ void __launch_bounds__(384) tc_prep_kernel(const float *__restrict__ 
                                                       const long long *__restrict__ row_index, long long R,
                                                       unsigned char *__restrict__ ctx, float *__restrict__ cx, long long Rp)
 {
-    constexpr int kPackCtas = kTrainStages * kPackSplit;
-    if ((int)blockIdx.x < kPackCtas) tc_pack_job(params, jobs.j[blockIdx.x / kPackSplit], (int)blockIdx.x % kPackSplit, pack);
-    else tc_ctx_tile((int)blockIdx.x - kPackCtas, x, cond, ld_cond, row_index, R, ctx, cx, Rp);
+    const int pack_ctas = jobs.n * kPackSplit;
+    if ((int)blockIdx.x < pack_ctas) tc_pack_job(params, jobs.j[blockIdx.x / kPackSplit], (int)blockIdx.x % kPackSplit, pack);
+    else tc_ctx_tile((int)blockIdx.x - pack_ctas, x, cond, ld_cond, row_index, R, ctx, cx, Rp);
+}
+
+// The handle's pack from the parameters mnle_create copied to the device (legacy default stream, waited for):
+// tc_rows_plan is the forward plan, tc_plan the same with every first layer replaced by the net's theta stage.
+int tc_handle_pack(Handle *H)
+{
+    TcPlan theta;
+    PackJobs jobs;
+    const size_t bytes = pack_plan(H->layout, true, &H->tc_rows_plan, &theta, &jobs);
+    H->tc_plan = H->tc_rows_plan;
+    for (TcStage &st : H->tc_plan.st)
+        if (st.kind == kStageInput) st = theta.st[st.net];
+    DDM_CUDA_TRY(cudaMalloc(&H->tc_pack, bytes));
+    tc_prep_kernel<<<(unsigned)(jobs.n * kPackSplit), 384>>>(H->params, jobs, static_cast<unsigned char *>(H->tc_pack), nullptr,
+                                                             nullptr, 0, nullptr, 0, nullptr, nullptr, 0);
+    DDM_CUDA_TRY(cudaGetLastError());
+    DDM_CUDA_TRY(cudaStreamSynchronize(0));
+    return DDM_OK;
 }
 
 static size_t train_pack_only_bytes(const Layout &L)
 {
-    return (train_plan(L, nullptr, nullptr, nullptr) + 127) / 128 * 128;
+    return (pack_plan(L, false, nullptr, nullptr, nullptr) + 127) / 128 * 128;
 }
 
 size_t tc_train_pack_bytes(int n_choices, long long R)
@@ -1218,11 +1133,10 @@ int tc_train_forward(const float *params_dev, const Layout &L, void *pack_dev, c
 {
     TcPlan plan;
     PackJobs jobs;
-    const size_t bytes = train_plan(L, &plan, nullptr, &jobs);
+    pack_plan(L, false, &plan, nullptr, &jobs);
     DDM_REQUIRE((reinterpret_cast<uintptr_t>(pack_dev) & 15u) == 0, "tc_train_forward: pack must be 16-byte aligned");
     unsigned char *ctx_dev = static_cast<unsigned char *>(pack_dev) + train_pack_only_bytes(L);
-    (void)bytes;
-    tc_prep_kernel<<<(unsigned)(kTrainStages * kPackSplit + (R + kTcM - 1) / kTcM), 384, 0, st>>>(
+    tc_prep_kernel<<<(unsigned)(jobs.n * kPackSplit + (R + kTcM - 1) / kTcM), 384, 0, st>>>(
         params_dev, jobs, static_cast<unsigned char *>(pack_dev), x_dev, cond_dev, ld_cond, row_index_dev, R, ctx_dev, dump.CX,
         dump.Rp);
     DDM_CUDA_TRY(cudaGetLastError());
@@ -1247,7 +1161,7 @@ int tc_train_forward(const float *params_dev, const Layout &L, void *pack_dev, c
 int tc_train_backward(const Layout &L, const void *pack_dev, long long R, const TcTrainDump &dump, cudaStream_t st)
 {
     TcPlan bplan;
-    train_plan(L, nullptr, &bplan, nullptr);
+    pack_plan(L, false, nullptr, &bplan, nullptr);
     int dev = 0, sms = 0, n_pairs = 0;
     long long grid = 0;
     DDM_CUDA_TRY(cudaGetDevice(&dev));
