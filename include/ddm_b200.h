@@ -346,6 +346,31 @@ int mnle_loglik_sum_batched_tc_f32(void *handle, const float *theta_dev, int64_t
                                    const float *pulses_dev, int64_t ld_pulses, int64_t D, int64_t T, int64_t C,
                                    float *out_dev, float *workspace_dev, void *stream);
 
+/*
+ * estimator.sample(sample_shape, condition) (sbi MixedDensityEstimator.sample): for each of B condition rows
+ * (cond_dev (B,85), row stride ld_cond) S draws of [rt seconds, choice].  x_out_dev (S,B,2) contiguous: sample s of
+ * condition b is row r = s*B + b.  The choice c is the smallest j with u_c < sum_{i<=j} softmax(logits)_i in fp64
+ * (K - 1 when rounding leaves u_c at or above the total); then u = n ~ N(0,1) goes through the ten spline transforms
+ * INVERTED, transform 9 first, each the identity outside [-10, 10] and located on the height knots inside, and
+ * rt = exp(mu_y + sigma_y * u).  The networks run on the tensor cores (the rows-mode tcgen05 forward, once for the
+ * categorical net and once for the ten conditioners on the sampled choice), the choice draw and the inverse chain
+ * in fp64.  rt is NOT clamped to the simulator's window: the estimator is a continuous density.
+ *   seed, sample_offset
+ *               native draws (draws_dev == NULL): one Philox4x32-10 block per row, key = (lo32(seed), hi32(seed)),
+ *               counter = (lo32(g), hi32(g), b, 0x4D4E4C45) for the global sample index g = sample_offset + s, so
+ *               splitting S over calls with matching offsets gives the bits of one call.  From its words w0..w3:
+ *                 u_c = (w0 + 0.5) * 2^-32
+ *                 u_1 = (((w1 >> 5) << 26 | (w2 >> 6)) + 0.5) * 2^-53
+ *                 n   = sqrt(-2 log u_1) * cos(pi * (w3 + 0.5) * 2^-31)            (fp64)
+ *   draws_dev   NULL, or (S*B, 2) fp32 [u_c in (0,1), n] per row, used INSTEAD of Philox.
+ * B*S <= 8e6 per call; workspace_dev 256-byte aligned with at least mnle_sample_tc_workspace_floats(K, B, S)
+ * floats (~3.7 KB per row; 0 when the shape is out of range).
+ */
+size_t mnle_sample_tc_workspace_floats(int n_choices, int64_t B, int64_t S);
+int mnle_sample_tc_f32(void *handle, const float *cond_dev, int64_t ld_cond, int64_t B, int64_t S,
+                       uint64_t seed, uint64_t sample_offset, const float *draws_dev,
+                       float *x_out_dev, float *workspace_dev, void *stream);
+
 /* ------------------------------------------------------------ MNLE training --- */
 
 /*

@@ -64,6 +64,8 @@ _SIGNATURES = {
     "mnle_loglik_sum_tc64_f32": (ctypes.c_int, [_ptr, _ptr, _i64, _ptr, _ptr, _i64, _i64, _i64, _ptr, _ptr, _ptr]),
     "mnle_loglik_grad_tc_workspace_floats": (ctypes.c_size_t, [_i32, _i64, _i64]),
     "mnle_loglik_sum_grad_tc_f32": (ctypes.c_int, [_ptr, _ptr, _i64, _ptr, _ptr, _i64, _i64, _i64, _ptr, _ptr, _ptr, _ptr]),
+    "mnle_sample_tc_workspace_floats": (ctypes.c_size_t, [_i32, _i64, _i64]),
+    "mnle_sample_tc_f32": (ctypes.c_int, [_ptr, _ptr, _i64, _i64, _i64, _u64, _u64, _ptr, _ptr, _ptr, _ptr]),
     "mnle_train_workspace_floats": (ctypes.c_size_t, [_i32, _i64]),
     "mnle_train_nll_grad_f32": (ctypes.c_int, [_ptr, _i32, _ptr, _ptr, _i64, _ptr, _i64, _ptr, _ptr, _ptr, _i32, _ptr]),
     "mnle_train_adam_f32": (ctypes.c_int, [_ptr, _ptr, _ptr, _ptr, _i32, _ptr, _f32, _f32, _f32, _f32, _i64, _f32, _ptr]),

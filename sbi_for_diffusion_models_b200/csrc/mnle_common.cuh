@@ -119,6 +119,10 @@ struct TcTrainDump {
     // of word c: column 32 c + j is negative) kept INSTEAD of the activations -- the backward-data pass needs nothing
     // else from a ReLU layer, and 16 bytes per (row, layer) replace 512.  The sigmoid layers still go through H.
     uint32_t *HM;
+    // forward only: the launch runs nets [net0, net0 + nets).  A launch with net0 > 0 rebuilds the context images but
+    // not the operand pack: a launch from net 0 in the same call must have written it (the sampler runs the
+    // categorical net, draws the choice into x, then runs the ten conditioners on the new context).
+    int net0 = 0, nets = kNets;
 };
 size_t tc_train_pack_bytes(int n_choices, long long R);  // operand pack + context images of R rows
 int tc_train_forward(const float *params_dev, const Layout &L, void *pack_dev, const float *x_dev, const float *cond_dev,

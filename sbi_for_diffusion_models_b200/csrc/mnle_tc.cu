@@ -449,13 +449,13 @@ static void tc_grid(long long n_tiles, int sms, int *n_pairs, long long *grid)
 // x 11 nets = 176 two-tile CTAs on 148 SMs, i.e. a second wave that is 19 % full and costs a whole pair time.
 // When the pairs that do not fit whole waves can run as ONE wave of one-tile CTAs instead, they do (13 pairs
 // + 6 singles per net: 143 + 66 CTAs; a single takes about 0.6 of a pair time).
-static void train_grid(long long n_tiles, int sms, int *n_pairs, long long *grid)
+static void train_grid(long long n_tiles, int sms, int *n_pairs, long long *grid, int nets = kNets)
 {
     long long pairs = n_tiles / 2;
-    const long long all = pairs * kNets, rem = all % sms;
+    const long long all = pairs * nets, rem = all % sms;
     if (all > sms && rem > 0) {
-        const long long fewer = (all - rem) / kNets;
-        if ((n_tiles - 2 * fewer) * kNets <= sms) pairs = fewer;
+        const long long fewer = (all - rem) / nets;
+        if ((n_tiles - 2 * fewer) * nets <= sms) pairs = fewer;
     }
     *n_pairs = (int)pairs;
     *grid = pairs + (n_tiles - 2 * pairs);
@@ -509,7 +509,7 @@ __global__ void __launch_bounds__(kTcThreads, 1)
     // more CTAs for a minibatch that is only a few dozen row tiles.  Barrier phases count local stages.
     // Training grids are (net, CTA of the net): CTAs are scheduled x-fastest, so every net's two-tile CTAs
     // start before any one-tile CTA does (see train_grid()).
-    const int net_id = (KEEP || BWD) ? (int)blockIdx.x : 0;
+    const int net_id = KEEP ? keep.net0 + (int)blockIdx.x : (BWD ? (int)blockIdx.x : 0);
     const int s_off = KEEP ? (net_id == 0 ? 0 : 4 + 3 * (net_id - 1)) : (BWD ? (net_id == 0 ? 0 : 3 + 2 * (net_id - 1)) : 0);
     const int n_st = KEEP ? (net_id == 0 ? 4 : 3) : (BWD ? (net_id == 0 ? 3 : 2) : kTcStages);
     // CTAs [0, n_pairs) take two tiles each, the rest one tile each (see tc_grid())
@@ -1135,6 +1135,8 @@ int tc_train_forward(const float *params_dev, const Layout &L, void *pack_dev, c
     PackJobs jobs;
     pack_plan(L, false, &plan, nullptr, &jobs);
     DDM_REQUIRE((reinterpret_cast<uintptr_t>(pack_dev) & 15u) == 0, "tc_train_forward: pack must be 16-byte aligned");
+    DDM_REQUIRE(dump.net0 >= 0 && dump.nets >= 1 && dump.net0 + dump.nets <= kNets, "tc_train_forward: bad net range");
+    if (dump.net0 > 0) jobs.n = 0;  // the pack was written by this call's launch from net 0: context images only
     unsigned char *ctx_dev = static_cast<unsigned char *>(pack_dev) + train_pack_only_bytes(L);
     tc_prep_kernel<<<(unsigned)(jobs.n * kPackSplit + (R + kTcM - 1) / kTcM), 384, 0, st>>>(
         params_dev, jobs, static_cast<unsigned char *>(pack_dev), x_dev, cond_dev, ld_cond, row_index_dev, R, ctx_dev, dump.CX,
@@ -1146,12 +1148,12 @@ int tc_train_forward(const float *params_dev, const Layout &L, void *pack_dev, c
     long long grid = 0;
     DDM_CUDA_TRY(cudaGetDevice(&dev));
     DDM_CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    train_grid((R + kTcM - 1) / kTcM, sms, &n_pairs, &grid);
+    train_grid((R + kTcM - 1) / kTcM, sms, &n_pairs, &grid, dump.nets);
     DDM_REQUIRE(grid <= 65535, "training minibatch too large for one launch (at most ~8e6 rows)");
     DDM_CUDA_TRY(cudaFuncSetAttribute(mnle_tc_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       (int)TcSmem<true>::kBytes));
     // (mu_y, sigma_y) sit at the tail of the parameter buffer: the kernel reads them through `hoist`
-    mnle_tc_kernel<true, true><<<dim3(kNets, (unsigned)grid), kTcThreads, TcSmem<true>::kBytes, st>>>(
+    mnle_tc_kernel<true, true><<<dim3((unsigned)dump.nets, (unsigned)grid), kTcThreads, TcSmem<true>::kBytes, st>>>(
         static_cast<const unsigned char *>(pack_dev), plan, cond_dev, ld_cond, x_dev, params_dev + L.mu_y, 1, 1, (int)R,
         n_pairs, 0.f, 1.f, L.n_choices, nullptr, nullptr, lp_dev, nullptr, row_index_dev, keep);
     DDM_CUDA_TRY(cudaGetLastError());

@@ -1091,6 +1091,9 @@ __device__ __forceinline__ void knots6_f64(const float (&logit)[kLaneBins], int 
     for (int i = 1; i < kLaneBins; ++i) lo[i] = hi[i - 1];
 }
 
+// INVERSE (the sampler): u <- spline^-1(u), the bin located on the height knots and the rational quadratic solved for
+// the position in the bin (nflows' rational_quadratic_spline(inverse=True)); logdet is not touched.
+template <bool INVERSE = false>
 __device__ __forceinline__ void rqs_quad_f64(double &u, double &logdet, const float *q, int base, int sub, bool live)
 {
     const double tail = (double)kTail;
@@ -1113,7 +1116,7 @@ __device__ __forceinline__ void rqs_quad_f64(double &u, double &logdet, const fl
     knots6_f64(qh, base, sub, hlo, hhi);
     int cnt = 0;
 #pragma unroll
-    for (int i = 0; i < kLaneBins; ++i) cnt += (ui >= wlo[i]) ? 1 : 0;
+    for (int i = 0; i < kLaneBins; ++i) cnt += (ui >= (INVERSE ? hlo[i] : wlo[i])) ? 1 : 0;
     const int b = quad_sum(cnt) - 1;
     const int sb = (b >= kLaneBins ? 1 : 0) + (b >= 2 * kLaneBins ? 1 : 0) + (b >= 3 * kLaneBins ? 1 : 0), ib = b - kLaneBins * sb;
     const double left = quad_get(pick6(wlo, ib), base, sb), right = quad_get(pick6(whi, ib), base, sb);
@@ -1125,6 +1128,15 @@ __device__ __forceinline__ void rqs_quad_f64(double &u, double &logdet, const fl
     const double d1 = (b == kBins - 1) ? 1.0 : 1e-3 + softplus_f((double)qd1);
     const double w = right - left, h = top - bottom;
     const double delta = h / w;
+    if (INVERSE) {
+        // a th^2 + b th + c = 0 for the position th in the bin; the root in [0, 1] in the cancellation-free form
+        const double i1 = d0 + d1 - 2.0 * delta, i2 = ui - bottom, i3 = i2 * i1;
+        const double qa = h * (delta - d0) + i3, qb = h * d0 - i3, qc = -delta * i2;
+        const double disc = fmax(qb * qb - 4.0 * qa * qc, 0.0);
+        const double root = (2.0 * qc) / (-qb - sqrt(disc));
+        if (inside) u = root * w + left;
+        return;
+    }
     const double th = (ui - left) / w;
     const double t1 = th * (1.0 - th);
     const double den = delta + (d0 + d1 - 2.0 * delta) * t1;
@@ -1227,6 +1239,153 @@ DDM_API int mnle_loglik_sum_tc64_f32(void *handle, const float *theta_dev, int64
                                                                                                   H->sigma_y, LP);
     DDM_CUDA_TRY(cudaGetLastError());
     precise_sum_kernel<<<(unsigned)((C + 127) / 128), 128, 0, st>>>(LP, (int)T, (int)C, out_dev);
+    DDM_CUDA_TRY(cudaGetLastError());
+    return DDM_OK;
+}
+
+// ---- estimator.sample: the choice from the categorical net, then log rt from the flow run in inverse --------------
+// sbi's MixedDensityEstimator.sample draws the choice first and then log rt from the spline flow conditioned on it.
+// Here: the S x B condition rows are expanded (row r = s * B + b), the tcgen05 rows-mode forward runs the categorical
+// net alone and keeps the logits, one thread per row draws the choice in fp64 and writes it into the context column,
+// the forward runs the ten conditioners on the new context and keeps the raw spline parameters, and four lanes per row
+// draw u from N(0, 1) and walk the ten splines backwards in fp64 (the same arithmetic as the tc64 potential).
+namespace mnle {
+
+constexpr uint32_t kSampleTag = 0x4D4E4C45u;  // counter word 3 of the sampler's Philox blocks (the simulator's is 0 or 1)
+
+__global__ void __launch_bounds__(256) sample_rows_kernel(const float *__restrict__ cond_in, long long ld_cond, long long B,
+                                                          long long R, float *__restrict__ cond, float *__restrict__ xr)
+{
+    const long long total = R * kCond;
+    for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long long)gridDim.x * blockDim.x) {
+        const long long r = idx / kCond;
+        const int j = (int)(idx - r * kCond);
+        cond[idx] = __ldg(cond_in + (r % B) * ld_cond + j);
+        if (j < 2) xr[2 * r + j] = j == 0 ? 1.0f : 0.0f;  // rt is not read by the forward; the choice starts at 0
+    }
+}
+
+// One Philox block per row (see the header): u_c from word 0, the normal from words 1-3 by Box-Muller in fp64.
+// draws != null: row r takes [u_c, n] = draws[2 r], draws[2 r + 1] instead.
+__global__ void __launch_bounds__(256) sample_choice_kernel(const float *__restrict__ LG, long long R, long long B, int n_choices,
+                                                            const ddm::PhiloxKey key, unsigned long long sample_offset,
+                                                            const float *__restrict__ draws, float *__restrict__ xr,
+                                                            double *__restrict__ normal)
+{
+    const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= R) return;
+    double uc, n;
+    if (draws != nullptr) {
+        uc = (double)__ldg(draws + 2 * r);
+        n = (double)__ldg(draws + 2 * r + 1);
+    } else {
+        const unsigned long long s = sample_offset + (unsigned long long)(r / B);
+        const uint32_t b = (uint32_t)(r % B);
+        uint32_t w[4];
+        ddm::philox4x32_10((uint32_t)s, (uint32_t)(s >> 32), b, kSampleTag, key, w);
+        uc = ((double)w[0] + 0.5) * 0x1p-32;
+        const double u1 = ((double)(((unsigned long long)(w[1] >> 5) << 26) | (w[2] >> 6)) + 0.5) * 0x1p-53;
+        n = sqrt(-2.0 * log(u1)) * cospi(((double)w[3] + 0.5) * 0x1p-31);
+    }
+    const float *lg = LG + (size_t)r * kMaxChoices;
+    double m = -INFINITY;
+    for (int j = 0; j < n_choices; ++j) m = fmax(m, (double)lg[j]);
+    double s = 0.0;
+    for (int j = 0; j < n_choices; ++j) s += exp((double)lg[j] - m);
+    int c = n_choices - 1;  // also when rounding leaves u_c at or above the last cumulative probability
+    double cum = 0.0;
+    for (int j = 0; j < n_choices - 1; ++j) {
+        cum += exp((double)lg[j] - m) / s;
+        if (uc < cum) {
+            c = j;
+            break;
+        }
+    }
+    xr[2 * r + 1] = (float)c;
+    normal[r] = n;
+}
+
+// (__maxnreg__: with only the launch bound ptxas settles on 64 registers and spills; 80 keeps three blocks per SM)
+__global__ void __maxnreg__(80) sample_chain_kernel(const float *__restrict__ Q, long long Rp, const float *__restrict__ xr,
+                                                                      const double *__restrict__ normal, long long R, float mu_y,
+                                                                      float sigma_y, float *__restrict__ x_out)
+{
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    const int sub = lane & (kRowLanes - 1), base = lane & ~(kRowLanes - 1), rw = lane / kRowLanes;
+    const long long row = ((long long)blockIdx.x * kRowWarps + wib) * kWarpRows + rw;
+    const bool live = row < R;
+    const long long rowc = live ? row : 0;
+    double u = live ? normal[rowc] : 0.0, unused = 0.0;
+#pragma unroll 1
+    for (int k = kTransforms - 1; k >= 0; --k) rqs_quad_f64<true>(u, unused, Q + ((size_t)k * Rp + rowc) * kQRows, base, sub, live);
+    if (sub == 0 && live) {
+        x_out[2 * row] = (float)exp((double)mu_y + (double)sigma_y * u);
+        x_out[2 * row + 1] = __ldg(xr + 2 * row + 1);
+    }
+}
+
+static size_t sample_floats(const Layout &L, long long R)
+{
+    const TrainDims d = train_dims(L, R);
+    auto up = [](size_t v) { return (v + 63) / 64 * 64; };
+    // operand pack + context images, spline parameters, logits | expanded condition rows | x rows | fp64 normals
+    return up(pack_floats(L, R) + (size_t)d.Rp * (kTransforms * kQRows + kMaxChoices)) + up((size_t)R * kCond) + up(2 * (size_t)R) +
+           2 * (size_t)d.Rp;
+}
+
+}  // namespace mnle
+
+DDM_API size_t mnle_sample_tc_workspace_floats(int n_choices, int64_t B, int64_t S)
+{
+    if (n_choices < 1 || n_choices > kMaxChoices || B <= 0 || S <= 0 || B * S > 8000000ll) return 0;
+    return sample_floats(make_layout(n_choices), B * S);
+}
+
+DDM_API int mnle_sample_tc_f32(void *handle, const float *cond_dev, int64_t ld_cond, int64_t B, int64_t S, uint64_t seed,
+                               uint64_t sample_offset, const float *draws_dev, float *x_out_dev, float *workspace_dev, void *stream)
+{
+    DDM_REQUIRE(B >= 0 && S >= 0, "mnle_sample_tc_f32: B=%lld S=%lld must not be negative", (long long)B, (long long)S);
+    DDM_REQUIRE(B == 0 || S <= 8000000ll / B, "mnle_sample_tc_f32: B=%lld x S=%lld rows (at most 8e6 per call)", (long long)B,
+                (long long)S);
+    DDM_REQUIRE(ld_cond >= kCond, "mnle_sample_tc_f32: ld_cond=%lld < 85", (long long)ld_cond);
+    const long long R = B * S;
+    if (R > 0) {
+        DDM_REQUIRE(cond_dev && x_out_dev && workspace_dev, "mnle_sample_tc_f32: null pointer");
+        DDM_REQUIRE((reinterpret_cast<uintptr_t>(workspace_dev) & 255u) == 0, "mnle_sample_tc_f32: workspace must be 256-byte aligned");
+    }
+    Handle *H = static_cast<Handle *>(handle);
+    if (H == nullptr || H->magic != kMagic) {
+        ddm::set_error("mnle_sample_tc_f32: bad handle");
+        return DDM_ERR_STATE;
+    }
+    if (R == 0) return DDM_OK;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const Layout &L = H->layout;
+    const TrainDims d = train_dims(L, R);
+    auto up = [](size_t v) { return (v + 63) / 64 * 64; };
+    float *pack = workspace_dev;
+    float *Q = pack + pack_floats(L, R);
+    float *LG = Q + (size_t)kTransforms * kQRows * d.Rp;
+    float *cond = workspace_dev + up(pack_floats(L, R) + (size_t)d.Rp * (kTransforms * kQRows + kMaxChoices));
+    float *xr = cond + up((size_t)R * kCond);
+    double *normal = reinterpret_cast<double *>(xr + up(2 * (size_t)R));
+    sample_rows_kernel<<<(unsigned)std::min<long long>((R * kCond + 255) / 256, 148 * 16), 256, 0, st>>>(cond_dev, (long long)ld_cond,
+                                                                                                        (long long)B, R, cond, xr);
+    DDM_CUDA_TRY(cudaGetLastError());
+    TcTrainDump keep{nullptr, Q, LG, d.Rp, nullptr, nullptr, nullptr};
+    keep.net0 = 0;
+    keep.nets = 1;  // the categorical net: logits
+    int rc = tc_train_forward(H->params, L, pack, xr, cond, (long long)kCond, nullptr, R, keep, nullptr, st);
+    if (rc != DDM_OK) return rc;
+    sample_choice_kernel<<<(unsigned)((R + 255) / 256), 256, 0, st>>>(LG, R, (long long)B, L.n_choices, ddm::make_philox_key(seed),
+                                                                     (unsigned long long)sample_offset, draws_dev, xr, normal);
+    DDM_CUDA_TRY(cudaGetLastError());
+    keep.net0 = 1;
+    keep.nets = kTransforms;  // the conditioners on [condition, sampled choice]: raw spline parameters
+    rc = tc_train_forward(H->params, L, pack, xr, cond, (long long)kCond, nullptr, R, keep, nullptr, st);
+    if (rc != DDM_OK) return rc;
+    sample_chain_kernel<<<(unsigned)((R + kBlockRows - 1) / kBlockRows), kRowWarps * 32, 0, st>>>(Q, d.Rp, xr, normal, R, H->mu_y,
+                                                                                                   H->sigma_y, x_out_dev);
     DDM_CUDA_TRY(cudaGetLastError());
     return DDM_OK;
 }

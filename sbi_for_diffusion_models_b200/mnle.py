@@ -178,3 +178,20 @@ def load_model(cfg=None, filename: str = "mnle_rt_choice.pt"):
     if "packed_params" in sd:
         return DeviceMNLE(PackedMNLE(sd["packed_params"].numpy(), int(sd["n_choices"])))
     return DeviceMNLE(PackedMNLE.from_state_dict(sd))      # a checkpoint written by sbi itself (see from_state_dict)
+
+
+@torch.no_grad()
+def posterior_predictive(density_estimator, theta: torch.Tensor, pulses: torch.Tensor, *, seed: Optional[int] = None
+                         ) -> torch.Tensor:
+    """One emulated session per parameter draw: theta (C,5) (e.g. from ``run_inference_mcmc``) and the session's pulse
+    trains (T,>=80) -> x (C,T,2) = [rt seconds, choice], x[c,t] drawn from the estimator at [theta_c, pulses_t].  One
+    ``sample`` call on the (C*T, 85) condition rows, row c*T + t; rt is not clamped (see ``DeviceMNLE.sample``)."""
+    est = as_device_estimator(density_estimator)
+    if theta.ndim != 2 or theta.shape[1] != 5:
+        raise ValueError(f"theta must be (C,5), got {tuple(theta.shape)}")
+    if pulses.ndim != 2 or pulses.shape[1] < 80:
+        raise ValueError(f"pulses must be (T,>=80), got {tuple(pulses.shape)}")
+    C, T = theta.shape[0], pulses.shape[0]
+    pl = pulses[:, :80].to(device=theta.device, dtype=torch.float32)
+    cond = torch.cat([theta.to(torch.float32)[:, None, :].expand(C, T, 5), pl[None, :, :].expand(C, T, 80)], dim=2)
+    return est.sample((), condition=cond.reshape(C * T, 85), seed=seed).reshape(C, T, 2)

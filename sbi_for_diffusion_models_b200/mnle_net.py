@@ -282,6 +282,65 @@ class DeviceMNLE(torch.nn.Module):
             _native.check(rc, "mnle_log_prob_rows")
         return out.to(condition.device).unsqueeze(0)
 
+    SAMPLE_MAX_ROWS = 8_000_000   # rows of one mnle_sample_tc_f32 call
+
+    def sample(self, sample_shape=torch.Size(), condition: Optional[torch.Tensor] = None, *, seed: Optional[int] = None,
+               draws: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """estimator.sample(sample_shape, condition): condition (B,85) -> x (*sample_shape, B, 2) = [rt seconds, choice]
+        on the condition's device.  The choice is drawn from the categorical net, then log rt from the spline flow
+        conditioned on it (the ten splines run in inverse, in fp64, on tensor-core network outputs).  rt is not clamped
+        to the simulator's window: the estimator is a continuous density, and sbi does not clamp its samples either.
+
+        [UNVERIFIED against sbi] the order "choice first, then the flow given the choice" and the output shape of sbi
+        >= 0.23's ConditionalDensityEstimator.sample follow sbi's MixedDensityEstimator; sbi is not installable where
+        this package is built, so they have not been checked against it (the inverse spline itself is pinned against
+        nflows' formulas, tests/test_mnle_sample_spec.py).
+
+        ``seed``: Philox key of the draws; None draws one from torch's global generator, so ``torch.manual_seed``
+        makes runs reproducible.  Sample s of condition b uses the Philox block of (s, b) (include/ddm_b200.h), so the
+        result does not depend on how large requests are split over calls.  ``draws``: (S*B, 2) or (*sample_shape, B,
+        2) of [u_choice in (0,1), standard normal] used instead of Philox (row s*B + b)."""
+        if condition is None:
+            raise ValueError("sample needs a condition (B,85)")
+        shape = torch.Size(sample_shape)
+        S = int(np.prod(shape)) if len(shape) else 1
+        dev = self._dev(condition)
+        cond = condition.to(device=dev, dtype=torch.float32)
+        if cond.ndim != 2 or cond.shape[1] != COND_DIM:
+            raise ValueError(f"condition must be (B,{COND_DIM}), got {tuple(cond.shape)}")
+        if cond.stride(1) != 1:
+            cond = cond.contiguous()
+        B = cond.shape[0]
+        if B > self.SAMPLE_MAX_ROWS:
+            raise ValueError(f"at most {self.SAMPLE_MAX_ROWS} conditions per call, got {B}")
+        if draws is not None:
+            if draws.numel() != S * B * 2:
+                raise ValueError(f"draws must hold (S*B, 2) = ({S * B}, 2) values, got {tuple(draws.shape)}")
+            draws = draws.reshape(S * B, 2).to(device=dev, dtype=torch.float32).contiguous()
+            seed = 0
+        elif seed is None:
+            from .simulator import next_seed
+            seed = next_seed()
+        L = _native.lib()
+        out = torch.empty((S * B, 2), dtype=torch.float32, device=dev)
+        if S * B > 0:
+            step = max(1, self.SAMPLE_MAX_ROWS // B)
+            with torch.cuda.device(dev):
+                stream = torch.cuda.current_stream(dev).cuda_stream
+                ws = None
+                for s0 in range(0, S, step):
+                    sc = min(step, S - s0)
+                    n_ws = L.mnle_sample_tc_workspace_floats(self.packed.n_choices, B, sc)
+                    if ws is None or ws.numel() < n_ws:
+                        ws = torch.empty((n_ws,), dtype=torch.float32, device=dev)   # torch allocations are 512-byte aligned
+                    d = draws[s0 * B:(s0 + sc) * B] if draws is not None else None
+                    rc = L.mnle_sample_tc_f32(self.packed.handle(dev), cond.data_ptr(), cond.stride(0) if B > 1 else COND_DIM,
+                                              B, sc, ctypes.c_uint64(seed & (2**64 - 1)), ctypes.c_uint64(s0),
+                                              d.data_ptr() if d is not None else None, out[s0 * B:].data_ptr(), ws.data_ptr(),
+                                              stream)
+                    _native.check(rc, "mnle_sample_tc_f32")
+        return out.reshape(*shape, B, 2).to(condition.device)
+
     def loglik_sum(self, theta: torch.Tensor, x_o: torch.Tensor, pulses: torch.Tensor, *, kernel: str = "auto"
                    ) -> torch.Tensor:
         """out[c] = sum_t log p(x_o[t] | [theta[c], pulses[t]]): theta (C,5), x_o (T,2), pulses (T,>=80)."""
