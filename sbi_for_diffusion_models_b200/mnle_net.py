@@ -269,7 +269,7 @@ class DeviceMNLE(torch.nn.Module):
         cond = condition.to(device=dev, dtype=torch.float32)
         if cond.ndim != 2 or cond.shape[1] != COND_DIM or cond.shape[0] != xr.shape[0]:
             raise ValueError(f"condition must be (R,{COND_DIM}) with R={xr.shape[0]}, got {tuple(cond.shape)}")
-        if cond.stride(1) != 1:
+        if cond.stride(1) != 1 or cond.stride(0) < COND_DIM:    # (a broadcast row has row stride 0)
             cond = cond.contiguous()
         R = xr.shape[0]
         with torch.cuda.device(dev):
@@ -308,7 +308,7 @@ class DeviceMNLE(torch.nn.Module):
         cond = condition.to(device=dev, dtype=torch.float32)
         if cond.ndim != 2 or cond.shape[1] != COND_DIM:
             raise ValueError(f"condition must be (B,{COND_DIM}), got {tuple(cond.shape)}")
-        if cond.stride(1) != 1:
+        if cond.stride(1) != 1 or cond.stride(0) < COND_DIM:    # (a broadcast row has row stride 0)
             cond = cond.contiguous()
         B = cond.shape[0]
         if B > self.SAMPLE_MAX_ROWS:

@@ -48,13 +48,18 @@ def trained_net():
     return p, PackedMNLE(packed, K)
 
 
+def _make_net(kind):
+    """(fp32 spec params, float64 spec params, estimator, kind); "init-K8" is a default-init net with 8 choices."""
+    if kind == "trained":
+        p, packed = trained_net()
+        return p, ms.cast_params(p, torch.float64), DeviceMNLE(packed), kind
+    p = ms.init_params(0) if kind == "init" else ms.init_params(0, n_choices=int(kind[len("init-K"):]))
+    return p, ms.cast_params(p, torch.float64), DeviceMNLE(PackedMNLE.from_params(p)), kind
+
+
 @pytest.fixture(scope="module", params=["init", "trained"])
 def net(request):
-    if request.param == "init":
-        p = ms.init_params(0)
-        return p, ms.cast_params(p, torch.float64), DeviceMNLE(PackedMNLE.from_params(p)), "init"
-    p, packed = trained_net()
-    return p, ms.cast_params(p, torch.float64), DeviceMNLE(packed), "trained"
+    return _make_net(request.param)
 
 
 @pytest.mark.parametrize("kernel", ["tc", "simt", "precise"])
@@ -84,6 +89,9 @@ def test_rows_api_matches_spec(net, kernel):
     assert est.log_prob(x.cuda(), condition=cond.cuda(), kernel=kernel).is_cuda
     wide = torch.cat([cond, torch.zeros(R, 7)], dim=1).cuda()
     assert torch.equal(est.log_prob(x.cuda(), condition=wide[:, :85], kernel=kernel).cpu(), got)
+    one = cond[3:4].cuda()                                              # a broadcast row (row stride 0)
+    assert torch.equal(est.log_prob(x.cuda(), condition=one.expand(R, 85), kernel=kernel),
+                       est.log_prob(x.cuda(), condition=one.repeat(R, 1), kernel=kernel))
     for r in (1, 127, 129):                                             # ragged last tile
         assert torch.equal(est.log_prob(x[:r], condition=cond[:r], kernel=kernel)[0], got[0, :r])
 
@@ -277,6 +285,51 @@ def test_potential_gradient_matches_autograd_of_the_spec(net, T, C):
     assert ok, seen
 
 
+def _tail_session(p32, K):
+    """Observations in the spline tails and on the tail bound, each with every choice in [0, K): rt in {1e-6, 3e-5,
+    1e-3, 8, 50, 1e4}, the float32 rt nearest to exp(mu_y +- 10 sigma_y) and its two neighbours (u = (log rt - mu_y) /
+    sigma_y on +-10 as closely as float32 rt allows, and on both sides of it), and u = +-10 +- 1e-6."""
+    mu, sg = float(p32["flow.mu_y"]), float(p32["flow.sigma_y"])
+    rts = [1e-6, 3e-5, 1e-3, 8.0, 50.0, 1e4]
+    for edge in (10.0, -10.0):
+        r = np.float32(np.exp(mu + sg * edge))
+        rts += [r, np.nextafter(r, np.float32(np.inf)), np.nextafter(r, np.float32(0.0))]
+        rts += [np.exp(mu + sg * (edge + d)) for d in (1e-6, -1e-6)]
+    rt = np.repeat(np.array(rts, np.float32), K)
+    choice = np.tile(np.arange(K), len(rts)).astype(np.float32)
+    x = torch.from_numpy(np.stack([rt, choice], 1))
+    pulses = torch.from_numpy(orc.pulses_pcg64_c(*orc.pcg64_state(np.random.default_rng(77)), 0, x.shape[0], 80, 0.75))
+    return x, pulses
+
+
+def test_fp64_chain_potentials_at_the_spline_tails(net):
+    """The tc64 potential and the reverse-mode gradient on observations in the linear tails of the splines and on the
+    tail bound, against the float64 spec (value) and autograd of it (gradient), with the bounds of
+    test_potential_sum_matches_spec (tc64) and test_potential_gradient_matches_autograd_of_the_spec (reverse mode)."""
+    p32, p64, est, kind = net
+    x, pulses = _tail_session(p32, est.packed.n_choices)
+    T, C = x.shape[0], 64
+    theta = orc.prior_sample(C, seed=41)
+    xr, cond = ms.potential_rows(theta, x, pulses)
+    want_rows = ms.log_prob(p64, xr, cond).reshape(T, C)
+    want = want_rows.sum(0)
+    scale = torch.maximum(want.abs(), want_rows.abs().sum(0) / 10)
+    got = est.loglik_sum(theta, x, pulses, kernel="tc64").double()
+    e = float(((got - want).abs() / scale).max())
+    th64 = theta.double().requires_grad_(True)
+    (want_grad,) = torch.autograd.grad(ms.loglik_sum(p64, th64, x, pulses).sum(), th64)
+    val, grad = est.loglik_sum_and_grad(theta, x, pulses, kernel="tc")
+    err_v = (val.double() - want).abs()
+    eg = (grad.double() - want_grad).abs() / (want_grad.abs() + 1e-2 * want_grad.abs().max())
+    # measured on a B200: tc64 1.9e-7 (init) and 5.1e-7 (trained) of scale; reverse mode value 4e-7 / 7e-6 relative,
+    # gradient median 1.3e-5 / 2.8e-5, mean 2.8e-4 / 1.2e-4, max 1.7e-2 / 5.6e-3
+    print(f"\n{kind}: T={T} tail trials: tc64 {e:.3g} of scale; reverse mode value {float((err_v / want.abs()).max()):.3g} "
+          f"relative, gradient median {float(eg.median()):.3g} mean {float(eg.mean()):.3g} max {float(eg.max()):.3g}")
+    assert e < (1e-4 if kind == "init" else 5e-4), e
+    assert bool((err_v <= (1e-4 if kind == "init" else 1e-3) * want.abs() + (2e-3 if kind == "init" else 2e-2)).all())
+    assert float(eg.median()) < 5e-3 and float(eg.mean()) < 5e-2 and float(eg.max()) < 5.0
+
+
 def test_sbc_sessions_one_launch_matches_per_dataset_calls():
     from sbi_for_diffusion_models_b200.sbc import simulate_sbc_sessions
     from sbi_for_diffusion_models_b200.simulator import simulate_trials
@@ -294,11 +347,18 @@ def test_sbc_sessions_one_launch_matches_per_dataset_calls():
     assert torch.equal(x2, x[2:])
 
 
-def test_outputs_and_workspaces_stay_in_bounds(net, monkeypatch):
+@pytest.fixture(scope="module", params=["init", "trained", "init-K8"])
+def bounds_net(request):
+    return _make_net(request.param)
+
+
+def test_outputs_and_workspaces_stay_in_bounds(bounds_net, monkeypatch):
     """Guard bands around every float32 device buffer the wrappers hand to the library (outputs and
-    workspaces of exactly the advertised size): ragged tiles must not write past either end.
+    workspaces of exactly the advertised size): ragged tiles must not write past either end.  The number of
+    choices changes the layout and the workspace sizes, so a net with 8 runs too.
     (compute-sanitizer is not available on the GPU pool, so the bounds are checked this way.)"""
-    _, _, est, _ = net
+    _, _, est, _ = bounds_net
+    K = est.packed.n_choices
     real_empty, bands, G = torch.empty, [], 2048
 
     def guarded(*size, **kw):
@@ -316,17 +376,23 @@ def test_outputs_and_workspaces_stay_in_bounds(net, monkeypatch):
     for R in (1, 127, 129, 3000):
         theta = orc.prior_sample(R, seed=2)
         pulses = torch.from_numpy(orc.pulses_pcg64_c(*orc.pcg64_state(np.random.default_rng(1)), 0, R, 80, 0.75))
-        x = torch.from_numpy(np.stack([np.exp(rs.uniform(-3, 2.1, R)), rs.randint(0, 3, R)], 1).astype(np.float32))
-        for kernel in ("tc", "simt"):
+        x = torch.from_numpy(np.stack([np.exp(rs.uniform(-3, 2.1, R)), rs.randint(0, K, R)], 1).astype(np.float32))
+        for kernel in ("tc", "simt", "precise"):
             assert bool(torch.isfinite(est.log_prob(x.cuda(), condition=torch.cat([theta, pulses], 1).cuda(), kernel=kernel)).all())
     for T, C in [(1, 1), (65, 7), (3, 300), (50, 130), (200, 33)]:
         x_o, pulses = _session(T)
+        if K != 3:
+            x_o[:, 1] = torch.from_numpy(rs.randint(0, K, T).astype(np.float32))
         theta = orc.prior_sample(C, seed=T)
-        for kernel in ("tc", "simt"):
+        for kernel in ("tc", "simt", "tc64", "precise"):
             assert bool(torch.isfinite(est.loglik_sum(theta.cuda(), x_o.cuda(), pulses.cuda(), kernel=kernel)).all())
-        if T * C < 2000:
-            out, grad = est.loglik_sum_and_grad(theta.cuda(), x_o.cuda(), pulses.cuda())
-            assert bool(torch.isfinite(out).all()) and bool(torch.isfinite(grad).all())
+        out, grad = est.loglik_sum_and_grad(theta.cuda(), x_o.cuda(), pulses.cuda(), kernel="tc")   # up to 6600 rows
+        assert bool(torch.isfinite(out).all()) and bool(torch.isfinite(grad).all())
+    for B, S in [(1, 1), (1, 127), (129, 1), (127, 3), (1000, 3)]:
+        cond = torch.cat([orc.prior_sample(B, seed=S), _session(B)[1]], 1).cuda()
+        for kw in ({"seed": 3}, {"draws": torch.from_numpy(np.stack([rs.uniform(0, 1, B * S), rs.standard_normal(B * S)], 1))}):
+            x = est.sample((S,), condition=cond, **kw)
+            assert bool(torch.isfinite(x).all()) and bool((x[..., 0] > 0).all())
     for D, T, C in [(3, 5, 130), (2, 1, 1), (4, 50, 37)]:
         xs, ps = zip(*[_session(T, seed=d) for d in range(D)])
         theta = orc.prior_sample(D * C, seed=9).reshape(D, C, 5)
@@ -337,11 +403,12 @@ def test_outputs_and_workspaces_stay_in_bounds(net, monkeypatch):
         assert bool((big[:G] == 12345.0).all()) and bool((big[G + n:] == 12345.0).all()), n
 
 
-@pytest.mark.parametrize("K", [2, 5, 8])
+@pytest.mark.parametrize("K", [1, 2, 5, 8])
 def test_other_numbers_of_choice_categories(K):
     """The categorical head has as many outputs as the training set has distinct choices (sbi sizes it
     from the data): 2 when no trial was censored (the "Bernoulli" head of BASELINE.json), up to the
-    library's limit of 8.  Rows API, potential (both kernels) and the gradient kernel against the spec."""
+    library's limit of 8; 1 (every trial the same choice) is admitted too.  Rows API (three kernels), potential
+    (four kernels) and the gradient kernel against the spec."""
     p = ms.init_params(11 + K, n_choices=K)
     p64 = ms.cast_params(p, torch.float64)
     est = DeviceMNLE(PackedMNLE.from_params(p))
@@ -353,9 +420,12 @@ def test_other_numbers_of_choice_categories(K):
     rs = np.random.RandomState(K)
     x = torch.from_numpy(np.stack([np.exp(rs.uniform(-3, 2.1, R)), rs.randint(0, K, R)], 1).astype(np.float32))
     want = ms.log_prob(p64, x, cond)
-    for kernel, tol in (("simt", 2e-3), ("tc", 4e-3)):
+    for kernel, tol in (("simt", 2e-3), ("tc", 4e-3), ("precise", 2e-3)):
         got = est.log_prob(x.unsqueeze(0), condition=cond, kernel=kernel)[0].double()
+        print(f"\nK={K} rows {kernel}: max {float((got - want).abs().max()):.3g} mean {float((got - want).abs().mean()):.3g}")
         assert float((got - want).abs().max()) < tol, (kernel, float((got - want).abs().max()))
+        if kernel == "precise":   # (the bounds of test_rows_api_matches_spec)
+            assert float((got - want).abs().mean()) < 2e-5, float((got - want).abs().mean())
     T, C = 23, 130
     th = orc.prior_sample(C, seed=5)
     x_o, pl = x[:T], pulses[:T]
@@ -363,6 +433,12 @@ def test_other_numbers_of_choice_categories(K):
     for kernel in ("simt", "tc"):
         got = est.loglik_sum(th, x_o, pl, kernel=kernel).double()
         assert float(((got - want_sum).abs() / want_sum.abs()).max()) < 1e-4, kernel
+    xr, cr = ms.potential_rows(th, x_o, pl)
+    scale = torch.maximum(want_sum.abs(), ms.log_prob(p64, xr, cr).reshape(T, C).abs().sum(0) / 10)
+    for kernel in ("precise", "tc64"):   # (the init-net bound of test_potential_sum_matches_spec)
+        got = est.loglik_sum(th, x_o, pl, kernel=kernel).double()
+        print(f"K={K} potential {kernel}: {float(((got - want_sum).abs() / scale).max()):.3g} of scale")
+        assert float(((got - want_sum).abs() / scale).max()) < 1e-4, (kernel, float(((got - want_sum).abs() / scale).max()))
     th64 = th[:9].double().requires_grad_(True)
     (want_grad,) = torch.autograd.grad(ms.loglik_sum(p64, th64, x_o, pl).sum(), th64)
     val, grad = est.loglik_sum_and_grad(th[:9], x_o, pl)
