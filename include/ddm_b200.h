@@ -315,8 +315,7 @@ int mnle_loglik_sum_grad_f32(void *handle, const float *theta_dev, int64_t ld_th
  * forward with activations kept, the per-row spline sweep, the tcgen05 backward-data pass, and the five theta
  * columns of every first layer are contracted and summed over the trials in a fixed order.  Same arguments as
  * mnle_loglik_sum_grad_f32; T*C <= 8e6 rows; workspace_dev 256-byte aligned with at least
- * mnle_loglik_grad_tc_workspace_floats(n_choices, T, C) floats (~38 KB per row: it holds the training step's buffers,
- * so 8e6 rows need ~286 GiB and a 180 GB B200 fits about 4.4e6).
+ * mnle_loglik_grad_tc_workspace_floats(n_choices, T, C) floats (~6.2 KB per row: ~46 GiB at 8e6 rows).
  */
 size_t mnle_loglik_grad_tc_workspace_floats(int n_choices, int64_t T, int64_t C);
 int mnle_loglik_sum_grad_tc_f32(void *handle, const float *theta_dev, int64_t ld_theta, const float *x_dev,

@@ -133,6 +133,18 @@ int tc_train_forward(const float *params_dev, const Layout &L, void *pack_dev, c
 int tc_train_backward(const Layout &L, const void *pack_dev, long long R, const TcTrainDump &dump, cudaStream_t st);
 constexpr uint32_t kMagic = 0x4D4E4C45u;  // "MNLE"
 
+// `handle` as a live MNLE handle (that also has its tensor-core operand pack when need_tc_pack), or null after setting
+// the error string "<entry point>: bad handle"; the entry point then returns DDM_ERR_STATE.
+inline Handle *live_handle(void *handle, const char *entry, bool need_tc_pack = false)
+{
+    Handle *H = static_cast<Handle *>(handle);
+    if (H == nullptr || H->magic != kMagic || (need_tc_pack && H->tc_pack == nullptr)) {
+        ddm::set_error("%s: bad handle", entry);
+        return nullptr;
+    }
+    return H;
+}
+
 __device__ __forceinline__ float softplus_f(float x)
 {
     return x > 20.0f ? x : log1pf(expf(x));  // torch.nn.functional.softplus, threshold 20

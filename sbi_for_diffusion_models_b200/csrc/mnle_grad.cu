@@ -298,11 +298,8 @@ DDM_API int mnle_loglik_sum_grad_f32(void *handle, const float *theta_dev, int64
                                      const float *pulses_dev, int64_t ld_pulses, int64_t T, int64_t C, float *out_dev,
                                      float *grad_dev, float *workspace_dev, void *stream)
 {
-    Handle *H = static_cast<Handle *>(handle);
-    if (H == nullptr || H->magic != kMagic) {
-        ddm::set_error("mnle_loglik_sum_grad_f32: bad handle");
-        return DDM_ERR_STATE;
-    }
+    Handle *H = live_handle(handle, "mnle_loglik_sum_grad_f32");
+    if (H == nullptr) return DDM_ERR_STATE;
     DDM_REQUIRE(T >= 0 && C >= 0 && C <= 65535 && T <= 0x7FFFFFFFll, "mnle_loglik_sum_grad: T=%lld C=%lld out of range",
                 (long long)T, (long long)C);
     if (C == 0) return DDM_OK;

@@ -117,13 +117,6 @@ __global__ void reduce_tiles_kernel(const float *__restrict__ partial, int n_til
     out[c] = s;
 }
 
-static Handle *check_handle(void *h)
-{
-    Handle *H = static_cast<Handle *>(h);
-    if (H == nullptr || H->magic != kMagic) return nullptr;
-    return H;
-}
-
 static int launch(Handle *H, const RowSource &src, dim3 grid, float *out, cudaStream_t st, bool precise = false)
 {
     static_assert(sizeof(SimtSmem) < 227 * 1024, "tile does not fit shared memory");
@@ -180,11 +173,8 @@ DDM_API int mnle_create(const float *packed_host, size_t n_floats, int n_choices
 
 DDM_API int mnle_destroy(void *handle)
 {
-    Handle *H = check_handle(handle);
-    if (H == nullptr) {
-        ddm::set_error("mnle_destroy: bad handle");
-        return DDM_ERR_STATE;
-    }
+    Handle *H = live_handle(handle, "mnle_destroy");
+    if (H == nullptr) return DDM_ERR_STATE;
     H->magic = 0;
     cudaFree(H->params);
     if (H->tc_pack) cudaFree(H->tc_pack);
@@ -195,11 +185,8 @@ DDM_API int mnle_destroy(void *handle)
 static int rows_impl(void *handle, const float *x_dev, const float *cond_dev, int64_t ld_cond, int64_t R, float *out_dev,
                      void *stream, bool precise)
 {
-    Handle *H = check_handle(handle);
-    if (H == nullptr) {
-        ddm::set_error("mnle_log_prob_rows_f32: bad handle");
-        return DDM_ERR_STATE;
-    }
+    Handle *H = live_handle(handle, "mnle_log_prob_rows_f32");
+    if (H == nullptr) return DDM_ERR_STATE;
     DDM_REQUIRE(R >= 0 && R <= 0x7FFFFFFFll * kTM, "mnle_log_prob_rows_f32: bad R");
     if (R == 0) return DDM_OK;
     DDM_REQUIRE(x_dev && cond_dev && out_dev, "mnle_log_prob_rows_f32: null pointer");
@@ -235,11 +222,8 @@ static int loglik_sum_impl(void *handle, const float *theta_dev, int64_t ld_thet
                            const float *pulses_dev, int64_t ld_pulses, int64_t T, int64_t C, float *out_dev,
                            float *workspace_dev, void *stream, bool precise)
 {
-    Handle *H = check_handle(handle);
-    if (H == nullptr) {
-        ddm::set_error("mnle_loglik_sum_simt_f32: bad handle");
-        return DDM_ERR_STATE;
-    }
+    Handle *H = live_handle(handle, "mnle_loglik_sum_simt_f32");
+    if (H == nullptr) return DDM_ERR_STATE;
     DDM_REQUIRE(T >= 0 && C >= 0 && C <= 65535 && T <= 0x7FFFFFFFll, "mnle_loglik_sum: T=%lld C=%lld out of range",
                 (long long)T, (long long)C);
     if (C == 0) return DDM_OK;

@@ -1232,11 +1232,8 @@ DDM_API int mnle_loglik_sum_batched_tc_f32(void *handle, const float *theta_dev,
                                            const float *pulses_dev, int64_t ld_pulses, int64_t D, int64_t T, int64_t C,
                                            float *out_dev, float *workspace_dev, void *stream)
 {
-    Handle *H = static_cast<Handle *>(handle);
-    if (H == nullptr || H->magic != kMagic || H->tc_pack == nullptr) {
-        ddm::set_error("mnle_loglik_sum_tc: bad handle");
-        return DDM_ERR_STATE;
-    }
+    Handle *H = live_handle(handle, "mnle_loglik_sum_tc", true);
+    if (H == nullptr) return DDM_ERR_STATE;
     DDM_REQUIRE(D >= 0 && T >= 0 && C >= 0 && D <= 0x7FFFFFFFll && T <= 0x7FFFFFFFll && C <= 0x7FFFFFFFll - kTcM,
                 "mnle_loglik_sum_tc: D=%lld T=%lld C=%lld out of range", (long long)D, (long long)T, (long long)C);
     if (C == 0 || D == 0) return DDM_OK;
@@ -1285,11 +1282,8 @@ DDM_API int mnle_loglik_sum_tc_f32(void *handle, const float *theta_dev, int64_t
 DDM_API int mnle_log_prob_rows_tc_f32(void *handle, const float *x_dev, const float *cond_dev, int64_t ld_cond, int64_t R,
                                       float *out_dev, void *stream)
 {
-    Handle *H = static_cast<Handle *>(handle);
-    if (H == nullptr || H->magic != kMagic || H->tc_pack == nullptr) {
-        ddm::set_error("mnle_log_prob_rows_tc_f32: bad handle");
-        return DDM_ERR_STATE;
-    }
+    Handle *H = live_handle(handle, "mnle_log_prob_rows_tc_f32", true);
+    if (H == nullptr) return DDM_ERR_STATE;
     DDM_REQUIRE(R >= 0 && R <= 0x7FFFFFFFll - kTcM, "mnle_log_prob_rows_tc_f32: bad R");
     if (R == 0) return DDM_OK;
     DDM_REQUIRE(x_dev && cond_dev && out_dev, "mnle_log_prob_rows_tc_f32: null pointer");

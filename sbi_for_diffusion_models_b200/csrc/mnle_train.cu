@@ -38,8 +38,30 @@ constexpr int kMaxGroups = 8;      // partial-gradient slices = row splits of th
 constexpr int kWgRows = 64;        // rows of the minibatch per chunk (= K of one accumulation step) of that kernel
 constexpr int kReduceThreads = 256;
 
+// Lays out a workspace from `base`: every buffer starts a multiple of 256 bytes past the base (enough for the 16-byte
+// bulk copies from the operand pack, the float4 stores into the spline parameters and the fp64 arrays), and floats()
+// is what the buffers handed out so far span.  A null base only counts.  Each entry point lays out its workspace in one
+// function that runs twice, on a null base for its *_workspace_floats query and on the caller's pointer in the
+// launcher, so the size a caller allocates and the buffers the launcher hands out cannot disagree.
+class Carver {
+  public:
+    explicit Carver(float *base) : base_(base) {}
+    template <typename T = float>
+    T *take(size_t n)
+    {
+        const size_t at = (used_ + 63) / 64 * 64;
+        used_ = at + (n * sizeof(T) + sizeof(float) - 1) / sizeof(float);
+        return base_ ? reinterpret_cast<T *>(base_ + at) : nullptr;
+    }
+    size_t floats() const { return used_; }
+
+  private:
+    float *base_;
+    size_t used_ = 0;
+};
+
 struct TrainBufs {
-    float *pack; // tensor-core operand pack of the current parameters (rebuilt every call)
+    unsigned char *pack; // tensor-core operand pack of the current parameters (rebuilt every call) + context images
     float *Q;    // [kTransforms][Rp][kQRows]  spline parameters -> their gradients
     float *LG;   // [Rp][kMaxChoices]          choice logits -> their gradients
     float *LP;   // [Rp]                       log p per row
@@ -68,28 +90,17 @@ static TrainDims train_dims(const Layout &L, long long R)
     return d;
 }
 
-static size_t pack_floats(const Layout &L, long long R)
-{
-    return (tc_train_pack_bytes(L.n_choices, R) + 63) / 64 * 16;  // whole 64-byte blocks, in floats
-}
-
-static size_t train_floats(const Layout &L, const TrainDims &d)
-{
-    return pack_floats(L, d.R) + (size_t)d.Rp * (kTransforms * kQRows + kMaxChoices + 1 + 2 * kNets * 3 * kHidden) + (size_t)d.groups * L.total +
-           (size_t)d.reduce_blocks;
-}
-
-static TrainBufs carve(float *ws, const Layout &L, const TrainDims &d)
+static TrainBufs train_workspace(Carver &ws, const Layout &L, const TrainDims &d)
 {
     TrainBufs b;
-    b.pack = ws;
-    b.Q = ws + pack_floats(L, d.R);
-    b.LG = b.Q + (size_t)kTransforms * kQRows * d.Rp;
-    b.LP = b.LG + (size_t)kMaxChoices * d.Rp;
-    b.H = b.LP + d.Rp;
-    b.DH = b.H + (size_t)kNets * 3 * kHidden * d.Rp;
-    b.P = b.DH + (size_t)kNets * 3 * kHidden * d.Rp;
-    b.SS = b.P + (size_t)d.groups * L.total;
+    b.pack = ws.take<unsigned char>(tc_train_pack_bytes(L.n_choices, d.R));
+    b.Q = ws.take((size_t)kTransforms * kQRows * d.Rp);
+    b.LG = ws.take((size_t)kMaxChoices * d.Rp);
+    b.LP = ws.take(d.Rp);
+    b.H = ws.take((size_t)kNets * 3 * kHidden * d.Rp);
+    b.DH = ws.take((size_t)kNets * 3 * kHidden * d.Rp);
+    b.P = ws.take((size_t)d.groups * L.total);
+    b.SS = ws.take(d.reduce_blocks);
     return b;
 }
 
@@ -783,7 +794,9 @@ DDM_API size_t mnle_train_workspace_floats(int n_choices, int64_t R)
 {
     if (n_choices < 1 || n_choices > kMaxChoices || R <= 0) return 0;
     const Layout L = make_layout(n_choices);
-    return train_floats(L, train_dims(L, R));
+    Carver ws(nullptr);
+    train_workspace(ws, L, train_dims(L, R));
+    return ws.floats();
 }
 
 DDM_API int mnle_train_nll_grad_f32(const float *params_dev, int n_choices, const float *x_dev, const float *cond_dev,
@@ -799,7 +812,8 @@ DDM_API int mnle_train_nll_grad_f32(const float *params_dev, int n_choices, cons
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const Layout L = make_layout(n_choices);
     const TrainDims d = train_dims(L, R);
-    const TrainBufs B = carve(workspace_dev, L, d);
+    Carver ws(workspace_dev);
+    const TrainBufs B = train_workspace(ws, L, d);
     TrainRows rows{x_dev, cond_dev, reinterpret_cast<const long long *>(row_index_dev), (long long)ld_cond, (long long)R};
 
     static_assert(sizeof(SimtSmem) < 113 * 1024, "two CTAs per SM");
@@ -954,18 +968,61 @@ __global__ void __launch_bounds__(128) potential_grad_final_kernel(const float *
     out[c] = sum;
 }
 
-static size_t potential_grad_floats(const Layout &L, long long T, long long C)
+// Only what the passes above read or write: no DH (the backward pass keeps no derivatives), no weight-gradient
+// partials, and activations of the categorical net's three sigmoid layers alone (the ReLU layers keep sign masks).
+struct PotentialGradBufs {
+    TrainBufs t;   // pack, Q, LG, LP; H, DH, P and SS stay null (train_rows_kernel reads only Q, LG and LP)
+    float *cond, *xr, *w1t, *gp, *part;
+    uint32_t *HM;  // [kNets][3][4][Rp] sign masks of the ReLU layers
+    float *H;      // [3][128][Rp] activations of the categorical net (net 0 of TcTrainDump::H)
+};
+
+static PotentialGradBufs potential_grad_workspace(Carver &ws, const Layout &L, const TrainDims &d, long long C)
 {
-    const long long R = T * C;
-    const TrainDims d = train_dims(L, R);
-    auto up = [](size_t v) { return (v + 63) / 64 * 64; };
-    size_t n = up(train_floats(L, d));
-    n += up((size_t)R * kCond) + up(2 * (size_t)R);         // the expanded rows
-    n += up((size_t)kNets * kHidden * 8);                   // theta columns of the first layers
-    n += up((size_t)kGradPlanes * 5 * (size_t)d.Rp);        // per-row partial gradients
-    n += up((size_t)kGradPlanes * (size_t)C * 5);           // per-chain partial gradients
-    n += (size_t)kNets * 3 * 4 * (size_t)d.Rp;              // sign masks of the ReLU layers
-    return n;
+    PotentialGradBufs b{};
+    b.t.pack = ws.take<unsigned char>(tc_train_pack_bytes(L.n_choices, d.R));
+    b.t.Q = ws.take((size_t)kTransforms * kQRows * d.Rp);
+    b.t.LG = ws.take((size_t)kMaxChoices * d.Rp);
+    b.t.LP = ws.take(d.Rp);
+    b.cond = ws.take((size_t)d.R * kCond);            // the expanded rows
+    b.xr = ws.take(2 * (size_t)d.R);
+    b.w1t = ws.take((size_t)kNets * kHidden * 8);       // theta columns of the first layers
+    b.gp = ws.take((size_t)kGradPlanes * 5 * (size_t)d.Rp);  // per-row partial gradients
+    b.part = ws.take((size_t)kGradPlanes * (size_t)C * 5);   // per-chain partial gradients
+    b.HM = ws.take<uint32_t>((size_t)kNets * 3 * 4 * (size_t)d.Rp);
+    // H last: the kernels address it as TcTrainDump::H, whose slots span all eleven nets, and only net 0's are carved.
+    // The ReLU nets keep sign masks in HM instead and the backward pass never reads their slots; were that wrong, their
+    // writes would land past the end of the workspace, where a guard band after the caller's buffer shows them.
+    b.H = ws.take((size_t)3 * kHidden * d.Rp);
+    return b;
+}
+
+// The argument checks and empty cases of the two potentials over expanded (trial, chain) rows.  *H is set when there
+// are rows to evaluate; otherwise the return value is final: an error, or DDM_OK when C == 0, or when T == 0 once out_dev
+// and (want_grad) grad_dev are zeroed.
+static int expanded_rows_prologue(const char *entry, Handle **H, void *handle, const float *theta_dev, int64_t ld_theta,
+                                  const float *x_dev, const float *pulses_dev, int64_t ld_pulses, int64_t T, int64_t C,
+                                  float *out_dev, bool want_grad, float *grad_dev, const float *workspace_dev,
+                                  cudaStream_t st)
+{
+    *H = nullptr;
+    Handle *h = live_handle(handle, entry);
+    if (h == nullptr) return DDM_ERR_STATE;
+    DDM_REQUIRE(T >= 0 && C >= 0 && T * C <= 8000000ll, "%s: T=%lld x C=%lld rows (at most 8e6 per call)", entry, (long long)T,
+                (long long)C);
+    if (C == 0) return DDM_OK;
+    DDM_REQUIRE(out_dev && (grad_dev || !want_grad), "%s: null output", entry);
+    if (T == 0) {
+        DDM_CUDA_TRY(cudaMemsetAsync(out_dev, 0, (size_t)C * sizeof(float), st));
+        if (want_grad) DDM_CUDA_TRY(cudaMemsetAsync(grad_dev, 0, (size_t)C * 5 * sizeof(float), st));
+        return DDM_OK;
+    }
+    DDM_REQUIRE(theta_dev && x_dev && pulses_dev && workspace_dev, "%s: null pointer", entry);
+    DDM_REQUIRE(ld_theta >= 5 && ld_pulses >= kCond - 5, "%s: ld_theta=%lld ld_pulses=%lld too small", entry, (long long)ld_theta,
+                (long long)ld_pulses);
+    DDM_REQUIRE((reinterpret_cast<uintptr_t>(workspace_dev) & 255u) == 0, "%s: workspace must be 256-byte aligned", entry);
+    *H = h;
+    return DDM_OK;
 }
 
 }  // namespace mnle
@@ -973,64 +1030,47 @@ static size_t potential_grad_floats(const Layout &L, long long T, long long C)
 DDM_API size_t mnle_loglik_grad_tc_workspace_floats(int n_choices, int64_t T, int64_t C)
 {
     if (n_choices < 1 || n_choices > kMaxChoices || T <= 0 || C <= 0) return 0;
-    return potential_grad_floats(make_layout(n_choices), T, C);
+    const Layout L = make_layout(n_choices);
+    Carver ws(nullptr);
+    potential_grad_workspace(ws, L, train_dims(L, T * C), C);
+    return ws.floats();
 }
 
 DDM_API int mnle_loglik_sum_grad_tc_f32(void *handle, const float *theta_dev, int64_t ld_theta, const float *x_dev,
                                         const float *pulses_dev, int64_t ld_pulses, int64_t T, int64_t C, float *out_dev,
                                         float *grad_dev, float *workspace_dev, void *stream)
 {
-    Handle *H = static_cast<Handle *>(handle);
-    if (H == nullptr || H->magic != kMagic) {
-        ddm::set_error("mnle_loglik_sum_grad_tc_f32: bad handle");
-        return DDM_ERR_STATE;
-    }
-    DDM_REQUIRE(T >= 0 && C >= 0 && T * C <= 8000000ll, "mnle_loglik_sum_grad_tc_f32: T=%lld x C=%lld rows (at most 8e6 per call)",
-                (long long)T, (long long)C);
-    if (C == 0) return DDM_OK;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    DDM_REQUIRE(out_dev && grad_dev, "mnle_loglik_sum_grad_tc_f32: null output");
-    if (T == 0) {
-        DDM_CUDA_TRY(cudaMemsetAsync(out_dev, 0, (size_t)C * sizeof(float), st));
-        DDM_CUDA_TRY(cudaMemsetAsync(grad_dev, 0, (size_t)C * 5 * sizeof(float), st));
-        return DDM_OK;
-    }
-    DDM_REQUIRE(theta_dev && x_dev && pulses_dev && workspace_dev, "mnle_loglik_sum_grad_tc_f32: null pointer");
-    DDM_REQUIRE(ld_theta >= 5 && ld_pulses >= kCond - 5, "mnle_loglik_sum_grad_tc_f32: ld_theta=%lld ld_pulses=%lld too small",
-                (long long)ld_theta, (long long)ld_pulses);
-    DDM_REQUIRE((reinterpret_cast<uintptr_t>(workspace_dev) & 255u) == 0, "mnle_loglik_sum_grad_tc_f32: workspace must be 256-byte aligned");
+    Handle *H;
+    int rc = expanded_rows_prologue("mnle_loglik_sum_grad_tc_f32", &H, handle, theta_dev, ld_theta, x_dev, pulses_dev, ld_pulses,
+                                    T, C, out_dev, true, grad_dev, workspace_dev, st);
+    if (H == nullptr) return rc;
     const Layout &L = H->layout;
     const long long R = T * C;
     const TrainDims d = train_dims(L, R);
-    const TrainBufs B = carve(workspace_dev, L, d);
-    auto up = [](size_t v) { return (v + 63) / 64 * 64; };
-    float *cond = workspace_dev + up(train_floats(L, d));
-    float *xr = cond + up((size_t)R * kCond);
-    float *w1t = xr + up(2 * (size_t)R);
-    float *gp = w1t + up((size_t)kNets * kHidden * 8);
-    float *part = gp + up((size_t)kGradPlanes * 5 * (size_t)d.Rp);
-    uint32_t *hm = reinterpret_cast<uint32_t *>(part + up((size_t)kGradPlanes * (size_t)C * 5));
-    potential_w1_kernel<<<kNets, kHidden, 0, st>>>(H->params, L, w1t);
+    Carver ws(workspace_dev);
+    const PotentialGradBufs B = potential_grad_workspace(ws, L, d, C);
+    potential_w1_kernel<<<kNets, kHidden, 0, st>>>(H->params, L, B.w1t);
     DDM_CUDA_TRY(cudaGetLastError());
     potential_rows_kernel<<<(unsigned)std::min<long long>((R * kCond + 255) / 256, 148 * 16), 256, 0, st>>>(
-        theta_dev, ld_theta, x_dev, pulses_dev, ld_pulses, (int)T, (int)C, cond, xr);
+        theta_dev, ld_theta, x_dev, pulses_dev, ld_pulses, (int)T, (int)C, B.cond, B.xr);
     DDM_CUDA_TRY(cudaGetLastError());
-    TrainRows rows{xr, cond, nullptr, (long long)kCond, R};
-    const TcTrainDump keep{B.H, B.Q, B.LG, d.Rp, nullptr, nullptr, nullptr, nullptr, nullptr, hm};
-    int rc = tc_train_forward(H->params, L, B.pack, xr, cond, (long long)kCond, nullptr, R, keep, B.LP, st);
+    TrainRows rows{B.xr, B.cond, nullptr, (long long)kCond, R};
+    const TcTrainDump keep{B.H, B.t.Q, B.t.LG, d.Rp, nullptr, nullptr, nullptr, nullptr, nullptr, B.HM};
+    rc = tc_train_forward(H->params, L, B.t.pack, B.xr, B.cond, (long long)kCond, nullptr, R, keep, B.t.LP, st);
     if (rc != DDM_OK) return rc;
     // scale = +1: the "loss" is the sum of the rows' log-probabilities
-    train_rows_kernel<<<(unsigned)((d.Rp + kBlockRows - 1) / kBlockRows), kRowWarps * 32, 0, st>>>(H->params, L, rows, d.Rp, 1.0f, 1, B);
+    train_rows_kernel<<<(unsigned)((d.Rp + kBlockRows - 1) / kBlockRows), kRowWarps * 32, 0, st>>>(H->params, L, rows, d.Rp, 1.0f, 1, B.t);
     DDM_CUDA_TRY(cudaGetLastError());
     // backward-data on tcgen05 without keeping the derivatives: the last epilogue of every net contracts d log p /
     // d (first-layer pre-activations) with the five theta columns of that layer and leaves five numbers per row
-    const TcTrainDump bwd{B.H, B.Q, B.LG, d.Rp, nullptr, nullptr, nullptr, gp, w1t, hm};
-    rc = tc_train_backward(L, B.pack, R, bwd, st);
+    const TcTrainDump bwd{B.H, B.t.Q, B.t.LG, d.Rp, nullptr, nullptr, nullptr, B.gp, B.w1t, B.HM};
+    rc = tc_train_backward(L, B.t.pack, R, bwd, st);
     if (rc != DDM_OK) return rc;
     const unsigned cb = (unsigned)((C + 127) / 128);
-    potential_grad_partial_kernel<<<dim3(cb, kGradPlanes), 128, 0, st>>>(gp, d.Rp, (int)T, (int)C, part);
+    potential_grad_partial_kernel<<<dim3(cb, kGradPlanes), 128, 0, st>>>(B.gp, d.Rp, (int)T, (int)C, B.part);
     DDM_CUDA_TRY(cudaGetLastError());
-    potential_grad_final_kernel<<<cb, 128, 0, st>>>(part, B.LP, (int)T, (int)C, out_dev, grad_dev);
+    potential_grad_final_kernel<<<cb, 128, 0, st>>>(B.part, B.t.LP, (int)T, (int)C, out_dev, grad_dev);
     DDM_CUDA_TRY(cudaGetLastError());
     return DDM_OK;
 }
@@ -1178,14 +1218,25 @@ __global__ void __launch_bounds__(128) precise_sum_kernel(const double *__restri
     out[c] = (float)sum;
 }
 
-static size_t tc64_floats(const Layout &L, long long T, long long C)
+struct Tc64Bufs {
+    unsigned char *pack;
+    float *Q, *LG;
+    float *lp32;  // the forward kernel's own fp32 log-prob slot (unused here)
+    float *cond, *xr;
+    double *LP;
+};
+
+static Tc64Bufs tc64_workspace(Carver &ws, const Layout &L, const TrainDims &d)
 {
-    const long long R = T * C;
-    const TrainDims d = train_dims(L, R);
-    auto up = [](size_t v) { return (v + 63) / 64 * 64; };
-    // operand pack + spline parameters + logits (the head of the training workspace), the expanded rows, fp64 log-probs
-    return up(pack_floats(L, R) + (size_t)d.Rp * (kTransforms * kQRows + kMaxChoices + 1)) + up((size_t)R * kCond) + up(2 * (size_t)R) +
-           2 * (size_t)d.Rp;
+    Tc64Bufs b;
+    b.pack = ws.take<unsigned char>(tc_train_pack_bytes(L.n_choices, d.R));
+    b.Q = ws.take((size_t)kTransforms * kQRows * d.Rp);
+    b.LG = ws.take((size_t)kMaxChoices * d.Rp);
+    b.lp32 = ws.take(d.Rp);
+    b.cond = ws.take((size_t)d.R * kCond);
+    b.xr = ws.take(2 * (size_t)d.R);
+    b.LP = ws.take<double>(d.Rp);
+    return b;
 }
 
 }  // namespace mnle
@@ -1193,52 +1244,36 @@ static size_t tc64_floats(const Layout &L, long long T, long long C)
 DDM_API size_t mnle_loglik_tc64_workspace_floats(int n_choices, int64_t T, int64_t C)
 {
     if (n_choices < 1 || n_choices > kMaxChoices || T <= 0 || C <= 0) return 0;
-    return tc64_floats(make_layout(n_choices), T, C);
+    const Layout L = make_layout(n_choices);
+    Carver ws(nullptr);
+    tc64_workspace(ws, L, train_dims(L, T * C));
+    return ws.floats();
 }
 
 DDM_API int mnle_loglik_sum_tc64_f32(void *handle, const float *theta_dev, int64_t ld_theta, const float *x_dev,
                                      const float *pulses_dev, int64_t ld_pulses, int64_t T, int64_t C, float *out_dev,
                                      float *workspace_dev, void *stream)
 {
-    Handle *H = static_cast<Handle *>(handle);
-    if (H == nullptr || H->magic != kMagic) {
-        ddm::set_error("mnle_loglik_sum_tc64_f32: bad handle");
-        return DDM_ERR_STATE;
-    }
-    DDM_REQUIRE(T >= 0 && C >= 0 && T * C <= 8000000ll, "mnle_loglik_sum_tc64_f32: T=%lld x C=%lld rows (at most 8e6 per call)",
-                (long long)T, (long long)C);
-    if (C == 0) return DDM_OK;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    DDM_REQUIRE(out_dev != nullptr, "mnle_loglik_sum_tc64_f32: null output");
-    if (T == 0) {
-        DDM_CUDA_TRY(cudaMemsetAsync(out_dev, 0, (size_t)C * sizeof(float), st));
-        return DDM_OK;
-    }
-    DDM_REQUIRE(theta_dev && x_dev && pulses_dev && workspace_dev, "mnle_loglik_sum_tc64_f32: null pointer");
-    DDM_REQUIRE(ld_theta >= 5 && ld_pulses >= kCond - 5, "mnle_loglik_sum_tc64_f32: ld_theta=%lld ld_pulses=%lld too small",
-                (long long)ld_theta, (long long)ld_pulses);
-    DDM_REQUIRE((reinterpret_cast<uintptr_t>(workspace_dev) & 255u) == 0, "mnle_loglik_sum_tc64_f32: workspace must be 256-byte aligned");
+    Handle *H;
+    int rc = expanded_rows_prologue("mnle_loglik_sum_tc64_f32", &H, handle, theta_dev, ld_theta, x_dev, pulses_dev, ld_pulses, T,
+                                    C, out_dev, false, nullptr, workspace_dev, st);
+    if (H == nullptr) return rc;
     const Layout &L = H->layout;
     const long long R = T * C;
     const TrainDims d = train_dims(L, R);
-    auto up = [](size_t v) { return (v + 63) / 64 * 64; };
-    float *pack = workspace_dev;
-    float *Q = pack + pack_floats(L, R);
-    float *LG = Q + (size_t)kTransforms * kQRows * d.Rp;
-    float *lp32 = LG + (size_t)kMaxChoices * d.Rp;   // the forward kernel's own fp32 log-prob slot (unused here)
-    float *cond = workspace_dev + up(pack_floats(L, R) + (size_t)d.Rp * (kTransforms * kQRows + kMaxChoices + 1));
-    float *xr = cond + up((size_t)R * kCond);
-    double *LP = reinterpret_cast<double *>(xr + up(2 * (size_t)R));
+    Carver ws(workspace_dev);
+    const Tc64Bufs B = tc64_workspace(ws, L, d);
     potential_rows_kernel<<<(unsigned)std::min<long long>((R * kCond + 255) / 256, 148 * 16), 256, 0, st>>>(
-        theta_dev, ld_theta, x_dev, pulses_dev, ld_pulses, (int)T, (int)C, cond, xr);
+        theta_dev, ld_theta, x_dev, pulses_dev, ld_pulses, (int)T, (int)C, B.cond, B.xr);
     DDM_CUDA_TRY(cudaGetLastError());
-    const TcTrainDump keep{nullptr, Q, LG, d.Rp, nullptr, nullptr, nullptr};
-    const int rc = tc_train_forward(H->params, L, pack, xr, cond, (long long)kCond, nullptr, R, keep, lp32, st);
+    const TcTrainDump keep{nullptr, B.Q, B.LG, d.Rp, nullptr, nullptr, nullptr};
+    rc = tc_train_forward(H->params, L, B.pack, B.xr, B.cond, (long long)kCond, nullptr, R, keep, B.lp32, st);
     if (rc != DDM_OK) return rc;
-    precise_rows_kernel<<<(unsigned)((R + kBlockRows - 1) / kBlockRows), kRowWarps * 32, 0, st>>>(Q, LG, d.Rp, xr, R, L.n_choices, H->mu_y,
-                                                                                                  H->sigma_y, LP);
+    precise_rows_kernel<<<(unsigned)((R + kBlockRows - 1) / kBlockRows), kRowWarps * 32, 0, st>>>(B.Q, B.LG, d.Rp, B.xr, R, L.n_choices,
+                                                                                                  H->mu_y, H->sigma_y, B.LP);
     DDM_CUDA_TRY(cudaGetLastError());
-    precise_sum_kernel<<<(unsigned)((C + 127) / 128), 128, 0, st>>>(LP, (int)T, (int)C, out_dev);
+    precise_sum_kernel<<<(unsigned)((C + 127) / 128), 128, 0, st>>>(B.LP, (int)T, (int)C, out_dev);
     DDM_CUDA_TRY(cudaGetLastError());
     return DDM_OK;
 }
@@ -1324,13 +1359,23 @@ __global__ void __maxnreg__(80) sample_chain_kernel(const float *__restrict__ Q,
     }
 }
 
-static size_t sample_floats(const Layout &L, long long R)
+struct SampleBufs {
+    unsigned char *pack;
+    float *Q, *LG;
+    float *cond, *xr;  // expanded condition rows, x rows
+    double *normal;
+};
+
+static SampleBufs sample_workspace(Carver &ws, const Layout &L, const TrainDims &d)
 {
-    const TrainDims d = train_dims(L, R);
-    auto up = [](size_t v) { return (v + 63) / 64 * 64; };
-    // operand pack + context images, spline parameters, logits | expanded condition rows | x rows | fp64 normals
-    return up(pack_floats(L, R) + (size_t)d.Rp * (kTransforms * kQRows + kMaxChoices)) + up((size_t)R * kCond) + up(2 * (size_t)R) +
-           2 * (size_t)d.Rp;
+    SampleBufs b;
+    b.pack = ws.take<unsigned char>(tc_train_pack_bytes(L.n_choices, d.R));
+    b.Q = ws.take((size_t)kTransforms * kQRows * d.Rp);
+    b.LG = ws.take((size_t)kMaxChoices * d.Rp);
+    b.cond = ws.take((size_t)d.R * kCond);
+    b.xr = ws.take(2 * (size_t)d.R);
+    b.normal = ws.take<double>(d.Rp);
+    return b;
 }
 
 }  // namespace mnle
@@ -1338,7 +1383,10 @@ static size_t sample_floats(const Layout &L, long long R)
 DDM_API size_t mnle_sample_tc_workspace_floats(int n_choices, int64_t B, int64_t S)
 {
     if (n_choices < 1 || n_choices > kMaxChoices || B <= 0 || S <= 0 || B * S > 8000000ll) return 0;
-    return sample_floats(make_layout(n_choices), B * S);
+    const Layout L = make_layout(n_choices);
+    Carver ws(nullptr);
+    sample_workspace(ws, L, train_dims(L, B * S));
+    return ws.floats();
 }
 
 DDM_API int mnle_sample_tc_f32(void *handle, const float *cond_dev, int64_t ld_cond, int64_t B, int64_t S, uint64_t seed,
@@ -1353,38 +1401,30 @@ DDM_API int mnle_sample_tc_f32(void *handle, const float *cond_dev, int64_t ld_c
         DDM_REQUIRE(cond_dev && x_out_dev && workspace_dev, "mnle_sample_tc_f32: null pointer");
         DDM_REQUIRE((reinterpret_cast<uintptr_t>(workspace_dev) & 255u) == 0, "mnle_sample_tc_f32: workspace must be 256-byte aligned");
     }
-    Handle *H = static_cast<Handle *>(handle);
-    if (H == nullptr || H->magic != kMagic) {
-        ddm::set_error("mnle_sample_tc_f32: bad handle");
-        return DDM_ERR_STATE;
-    }
+    Handle *H = live_handle(handle, "mnle_sample_tc_f32");
+    if (H == nullptr) return DDM_ERR_STATE;
     if (R == 0) return DDM_OK;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const Layout &L = H->layout;
     const TrainDims d = train_dims(L, R);
-    auto up = [](size_t v) { return (v + 63) / 64 * 64; };
-    float *pack = workspace_dev;
-    float *Q = pack + pack_floats(L, R);
-    float *LG = Q + (size_t)kTransforms * kQRows * d.Rp;
-    float *cond = workspace_dev + up(pack_floats(L, R) + (size_t)d.Rp * (kTransforms * kQRows + kMaxChoices));
-    float *xr = cond + up((size_t)R * kCond);
-    double *normal = reinterpret_cast<double *>(xr + up(2 * (size_t)R));
+    Carver ws(workspace_dev);
+    const SampleBufs W = sample_workspace(ws, L, d);
     sample_rows_kernel<<<(unsigned)std::min<long long>((R * kCond + 255) / 256, 148 * 16), 256, 0, st>>>(cond_dev, (long long)ld_cond,
-                                                                                                        (long long)B, R, cond, xr);
+                                                                                                        (long long)B, R, W.cond, W.xr);
     DDM_CUDA_TRY(cudaGetLastError());
-    TcTrainDump keep{nullptr, Q, LG, d.Rp, nullptr, nullptr, nullptr};
+    TcTrainDump keep{nullptr, W.Q, W.LG, d.Rp, nullptr, nullptr, nullptr};
     keep.net0 = 0;
     keep.nets = 1;  // the categorical net: logits
-    int rc = tc_train_forward(H->params, L, pack, xr, cond, (long long)kCond, nullptr, R, keep, nullptr, st);
+    int rc = tc_train_forward(H->params, L, W.pack, W.xr, W.cond, (long long)kCond, nullptr, R, keep, nullptr, st);
     if (rc != DDM_OK) return rc;
-    sample_choice_kernel<<<(unsigned)((R + 255) / 256), 256, 0, st>>>(LG, R, (long long)B, L.n_choices, ddm::make_philox_key(seed),
-                                                                     (unsigned long long)sample_offset, draws_dev, xr, normal);
+    sample_choice_kernel<<<(unsigned)((R + 255) / 256), 256, 0, st>>>(W.LG, R, (long long)B, L.n_choices, ddm::make_philox_key(seed),
+                                                                     (unsigned long long)sample_offset, draws_dev, W.xr, W.normal);
     DDM_CUDA_TRY(cudaGetLastError());
     keep.net0 = 1;
     keep.nets = kTransforms;  // the conditioners on [condition, sampled choice]: raw spline parameters
-    rc = tc_train_forward(H->params, L, pack, xr, cond, (long long)kCond, nullptr, R, keep, nullptr, st);
+    rc = tc_train_forward(H->params, L, W.pack, W.xr, W.cond, (long long)kCond, nullptr, R, keep, nullptr, st);
     if (rc != DDM_OK) return rc;
-    sample_chain_kernel<<<(unsigned)((R + kBlockRows - 1) / kBlockRows), kRowWarps * 32, 0, st>>>(Q, d.Rp, xr, normal, R, H->mu_y,
+    sample_chain_kernel<<<(unsigned)((R + kBlockRows - 1) / kBlockRows), kRowWarps * 32, 0, st>>>(W.Q, d.Rp, W.xr, W.normal, R, H->mu_y,
                                                                                                    H->sigma_y, x_out_dev);
     DDM_CUDA_TRY(cudaGetLastError());
     return DDM_OK;

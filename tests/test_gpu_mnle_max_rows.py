@@ -7,9 +7,9 @@ spec, and bit for bit against small calls on the same rows (rows are independent
 trials run in a fixed order that does not depend on the other chains).
 
 Each test needs one large workspace (sample and tc64 potential ~27 GiB each at 8e6 rows, the reverse-mode gradient
-~38 KB per row: ~286 GiB at 8e6 rows, more than a 180 GB B200 has, so it also runs at 4e6 rows, ~143 GiB, where the
-byte offsets into its buffers are still past 2^32) and frees it before the next; a test skips, naming the amount,
-when the device has less free memory than that."""
+~6.2 KB per row: ~46 GiB at 8e6 rows; it also runs at 4e6 rows, ~23 GiB, where the byte offsets into its buffers are
+still past 2^32) and frees it before the next; a test skips, naming the amount, when the device has less free memory
+than that."""
 import gc
 import os
 
