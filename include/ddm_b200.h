@@ -347,6 +347,29 @@ int mnle_loglik_sum_batched_tc_f32(void *handle, const float *theta_dev, int64_t
                                    float *out_dev, float *workspace_dev, void *stream);
 
 /*
+ * D observed sessions of different lengths in one launch: session d owns the flat trials
+ * [trial_offsets[d], trial_offsets[d+1]) of x_dev (N,2) and pulses_dev (N,>=80, row stride ld_pulses);
+ * theta_dev (D*C,5) row stride ld_theta, out_dev (D*C,);
+ * out[d*C + c] = sum over the trials t of session d of log p(x[t] | [theta[d*C + c], pulses[t]]),
+ * 0 for an empty session.  Every output is the bits mnle_loglik_sum_tc_f32 gives for that session alone.
+ * trial_offsets_dev: DEVICE int64 (D+1,) with offsets[0] = 0, offsets[D] = N and offsets[d] <= offsets[d+1];
+ * the kernels do not check them (they would have to copy them to the host), the caller must.
+ * N <= 524280 per call; workspace_dev >= mnle_loglik_sessions_tc_workspace_floats(D,N,C) floats, 16-byte aligned.
+ */
+size_t mnle_loglik_sessions_tc_workspace_floats(int64_t D, int64_t N, int64_t C);
+int mnle_loglik_sum_sessions_tc_f32(void *handle, const float *theta_dev, int64_t ld_theta, const float *x_dev,
+                                    const float *pulses_dev, int64_t ld_pulses, const int64_t *trial_offsets_dev,
+                                    int64_t D, int64_t N, int64_t C, float *out_dev, float *workspace_dev, void *stream);
+/* The same ragged sessions on the _tc64 path (tensor-core networks, fp64 spline chain and fp64 sums over each
+ * session's trials in trial order); every output is the bits mnle_loglik_sum_tc64_f32 gives for that session
+ * alone.  N*C <= 8e6 and D <= 65535 per call; workspace_dev 256-byte aligned with at least
+ * mnle_loglik_sessions_tc64_workspace_floats(n_choices, D, N, C) floats. */
+size_t mnle_loglik_sessions_tc64_workspace_floats(int n_choices, int64_t D, int64_t N, int64_t C);
+int mnle_loglik_sum_sessions_tc64_f32(void *handle, const float *theta_dev, int64_t ld_theta, const float *x_dev,
+                                      const float *pulses_dev, int64_t ld_pulses, const int64_t *trial_offsets_dev,
+                                      int64_t D, int64_t N, int64_t C, float *out_dev, float *workspace_dev, void *stream);
+
+/*
  * estimator.sample(sample_shape, condition) (sbi MixedDensityEstimator.sample): for each of B condition rows
  * (cond_dev (B,85), row stride ld_cond) S draws of [rt seconds, choice].  x_out_dev (S,B,2) contiguous: sample s of
  * condition b is row r = s*B + b.  The choice c is the smallest j with u_c < sum_{i<=j} softmax(logits)_i in fp64

@@ -58,6 +58,12 @@ _SIGNATURES = {
     "mnle_loglik_sum_tc_f32": (ctypes.c_int, [_ptr, _ptr, _i64, _ptr, _ptr, _i64, _i64, _i64, _ptr, _ptr, _ptr]),
     "mnle_loglik_batched_tc_workspace_floats": (ctypes.c_size_t, [_i64, _i64, _i64]),
     "mnle_loglik_sum_batched_tc_f32": (ctypes.c_int, [_ptr, _ptr, _i64, _ptr, _ptr, _i64, _i64, _i64, _i64, _ptr, _ptr, _ptr]),
+    "mnle_loglik_sessions_tc_workspace_floats": (ctypes.c_size_t, [_i64, _i64, _i64]),
+    "mnle_loglik_sum_sessions_tc_f32": (ctypes.c_int, [_ptr, _ptr, _i64, _ptr, _ptr, _i64, _ptr, _i64, _i64, _i64, _ptr, _ptr,
+                                                       _ptr]),
+    "mnle_loglik_sessions_tc64_workspace_floats": (ctypes.c_size_t, [_i32, _i64, _i64, _i64]),
+    "mnle_loglik_sum_sessions_tc64_f32": (ctypes.c_int, [_ptr, _ptr, _i64, _ptr, _ptr, _i64, _ptr, _i64, _i64, _i64, _ptr,
+                                                         _ptr, _ptr]),
     "mnle_loglik_grad_workspace_floats": (ctypes.c_size_t, [_i64, _i64]),
     "mnle_loglik_sum_grad_f32": (ctypes.c_int, [_ptr, _ptr, _i64, _ptr, _ptr, _i64, _i64, _i64, _ptr, _ptr, _ptr, _ptr]),
     "mnle_loglik_tc64_workspace_floats": (ctypes.c_size_t, [_i32, _i64, _i64]),

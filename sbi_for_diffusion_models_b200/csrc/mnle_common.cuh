@@ -253,4 +253,17 @@ __device__ __forceinline__ Real categorical_logp(const float *logits, int ls, in
     return rlog(p);
 }
 
+// Session of flat trial t (0 <= t < offsets[D]) in a ragged batch: the d with offsets[d] <= t < offsets[d + 1].
+// Empty sessions (offsets[d] == offsets[d + 1]) own no trial and are never returned.
+__device__ __forceinline__ int session_of(const long long *__restrict__ offsets, int D, long long t)
+{
+    int lo = 0, hi = D;  // offsets[lo] <= t < offsets[hi]
+    while (hi - lo > 1) {
+        const int mid = (lo + hi) >> 1;
+        if (__ldg(offsets + mid) <= t) lo = mid;
+        else hi = mid;
+    }
+    return lo;
+}
+
 }  // namespace mnle

@@ -141,19 +141,31 @@ __global__ void __launch_bounds__(128) tc_selftest_kernel(const float *__restric
 // grid = (nets, ceil(T / 8)): the 128 x 81 weight block is staged in shared memory once per block
 // and reused for 8 trials.  Block (0, 0) also clears the per-chain-block arrival counters of the
 // fused kernel's final reduction.
+// SESS, ragged sessions (offsets: D + 1 entries, T = offsets[D] flat trials): the net-0 blocks also
+// write the session of each of their trials to sess[] (one binary search per trial instead of one per
+// tile and thread in the fused kernel), and write the C zeros of the empty sessions d = y (mod grid y)
+// -- such a session has no tile that could write them.
 constexpr int kHoistTrials = 8;
 constexpr int kHoistK = kCtx - 5;  // 81
+template <bool SESS>
 __global__ void __launch_bounds__(kHidden) mnle_hoist_kernel(const float *__restrict__ params, Layout L,
                                                             const float *__restrict__ x,
                                                             const float *__restrict__ pulses, long long ld_pulses, int T,
                                                             float *__restrict__ hoist, unsigned int *__restrict__ counters,
-                                                            int n_counters)
+                                                            int n_counters, const long long *__restrict__ offsets, int D,
+                                                            int C, int *__restrict__ sess, float *__restrict__ out)
 {
     __shared__ float w_s[kHidden * kHoistK];
     __shared__ float in_s[kHoistTrials][kHoistK + 3];
     const int net = blockIdx.x, t0 = blockIdx.y * kHoistTrials, j = threadIdx.x;
     if (blockIdx.x == 0 && blockIdx.y == 0)
         for (int i = j; i < n_counters; i += kHidden) counters[i] = 0u;
+    if (SESS && blockIdx.x == 0) {
+        if (j < kHoistTrials && t0 + j < T) sess[t0 + j] = session_of(offsets, D, t0 + j);
+        for (int d = blockIdx.y; d < D; d += gridDim.y)
+            if (__ldg(offsets + d + 1) == __ldg(offsets + d))
+                for (int c = j; c < C; c += kHidden) out[(size_t)d * C + c] = 0.f;
+    }
     const int K = net == 0 ? kCond : kCtx;
     const float *W = params + (net == 0 ? L.cat_W0 : L.fl_W1[net - 1]);
     // 81 independent loads per thread in flight (fully unrolled): the block is latency-bound
@@ -427,7 +439,9 @@ __device__ __forceinline__ void tc_epilogue_spline(uint32_t trow, const float *b
 }
 
 // tile = ((d * T + t) * CB + chain block), chain block fastest; grid: tc_grid().
-// D independent datasets (own x, pulses and C chains each) share one launch.
+// D independent datasets (own x, pulses and C chains each) share one launch.  SESS, ragged sessions
+// (a template flag, so that the uniform path's code is what it was): tile = (flat trial * CB + chain block), session d = sess[flat trial] (written by
+// mnle_hoist_kernel), whose T_d trials start at trial_offsets[d].
 // Launch shape of the potential kernel: whole waves of two-tile CTAs (one CTA per SM), and the tiles that
 // are left over once the last FULL wave of pairs is placed go one per CTA when that fits a single wave --
 // a half-empty wave of pairs costs a whole pair time (400 tiles on 148 SMs: 148 pairs + 104 singles
@@ -471,7 +485,7 @@ static void train_grid(long long n_tiles, int sms, int *n_pairs, long long *grid
 // BWD (rows layout, the training backward-data pass): the A image of a net's first stage holds the
 // gradient rows (d loss / d spline parameters or logits), the weight images are the transposed ones, and
 // every epilogue multiplies by the activation derivative (tc_epilogue_mask) and writes keep.DH.
-template <bool ROWS, bool KEEP = false, bool BWD = false, bool POT = false>
+template <bool ROWS, bool KEEP = false, bool BWD = false, bool POT = false, bool SESS = false>
 __global__ void __launch_bounds__(kTcThreads, 1)
     mnle_tc_kernel(const unsigned char *__restrict__ pack, const __grid_constant__ TcPlan plan,
                    const float *__restrict__ theta, long long ld_theta, const float *__restrict__ x,
@@ -479,11 +493,13 @@ __global__ void __launch_bounds__(kTcThreads, 1)
                    int n_choices,
                    float *__restrict__ partial, unsigned int *__restrict__ counters, float *__restrict__ out,
                    long long *__restrict__ trace, const long long *__restrict__ row_index = nullptr,
-                   TcTrainDump keep = TcTrainDump{})
+                   TcTrainDump keep = TcTrainDump{}, const int *__restrict__ sess = nullptr,
+                   const long long *__restrict__ trial_offsets = nullptr)
 {
     static_assert(ROWS || !KEEP, "only the rows-mode kernel keeps activations");
     static_assert(!BWD || (ROWS && !KEEP), "the backward pass uses the rows-mode layout");
     static_assert(!POT || BWD, "POT selects the potential-gradient flavour of the backward pass");
+    static_assert(!SESS || !ROWS, "ragged sessions are a potential-mode layout");
     extern __shared__ __align__(1024) unsigned char smem[];
     using SM = TcSmem<ROWS>;
     constexpr int kTcSlots = SM::kSlots;
@@ -637,7 +653,8 @@ __global__ void __launch_bounds__(kTcThreads, 1)
         // ====== epilogue warps: tile X, lane quarter q (thread = row), column half hf ==========
         const int X = (warp >> 2) & 1, q = warp & 3, hf = warp >> 3, r = 32 * q + lane;
         // t = flattened (dataset, trial) index, c = chain within the dataset
-        const int tile = tile0 + X, t = tile / CB, cb = tile - t * CB, d = t / T, c = cb * kTcM + r;
+        const int tile = tile0 + X, t = tile / CB, cb = tile - t * CB, c = cb * kTcM + r;
+        const int d = SESS ? __ldg(sess + t) : t / T;
         const bool live = c < C;
         const long long c_glob = (long long)d * C + c;
         const uint32_t trow = tmem + (uint32_t)X * kTmemTile + ((uint32_t)(32 * q) << 16);
@@ -879,19 +896,21 @@ __global__ void __launch_bounds__(kTcThreads, 1)
             if (!KEEP && !BWD && hf == 0 && live) out[c_glob] = lp + (-0.5f * u * u - 0.9189385332046727f) + logdet - y;
         } else if (hf == 0) {
             // ---- sum over trials, fixed order: the tile that arrives last at its chain block adds
-            // the T partial rows (every run gives the same bits whichever tile that is)
+            // the T_d partial rows of its session (every run gives the same bits whichever tile that is)
             if (live) partial[(size_t)t * C + c] = lp + (-0.5f * u * u - 0.9189385332046727f) + logdet - y;
+            const long long first = SESS ? __ldg(trial_offsets + d) : (long long)d * T;
+            const int Td = SESS ? (int)(__ldg(trial_offsets + d + 1) - first) : T;
             uint32_t *last_s = tmem_slot + 1 + X;
             __threadfence();
             asm volatile("bar.sync %0, 128;" ::"r"(1 + X) : "memory");
-            if (q == 0 && lane == 0) *last_s = (atomicAdd(&counters[d * CB + cb], 1u) == (unsigned)(T - 1));
+            if (q == 0 && lane == 0) *last_s = (atomicAdd(&counters[d * CB + cb], 1u) == (unsigned)(Td - 1));
             asm volatile("bar.sync %0, 128;" ::"r"(1 + X) : "memory");
             if (*last_s && live) {
                 __threadfence();
-                const float *col = partial + (size_t)d * T * C + c;
+                const float *col = partial + (size_t)first * C + c;
                 float sum = 0.f;
 #pragma unroll 10
-                for (int tt = 0; tt < T; ++tt) sum += __ldcg(col + (size_t)tt * C);
+                for (int tt = 0; tt < Td; ++tt) sum += __ldcg(col + (size_t)tt * C);
                 out[c_glob] = sum;
             }
         }
@@ -1217,10 +1236,77 @@ DDM_API int mnle_tc_set_trace(long long *trace_dev)
     return DDM_OK;
 }
 
+// Workspace of the fused potential over N flat trials of D datasets / sessions, in floats: the per-trial first
+// layers, the per-row partial sums, the arrival counters and (ragged sessions) the session of every trial.
+static size_t tc_sum_workspace(float *base, long long D, long long N, long long C, bool sessions, float **hoist,
+                               float **partial, unsigned int **counters, int **sess)
+{
+    const size_t n_hoist = (size_t)N * kNets * kHidden, n_partial = (size_t)N * (size_t)C;
+    const size_t n_counters = (size_t)D * (size_t)((C + kTcM - 1) / kTcM);
+    if (base != nullptr) {
+        *hoist = base;
+        *partial = base + n_hoist;
+        *counters = reinterpret_cast<unsigned int *>(*partial + n_partial);
+        *sess = sessions ? reinterpret_cast<int *>(base + n_hoist + n_partial + n_counters) : nullptr;
+    }
+    return n_hoist + n_partial + n_counters + (sessions ? (size_t)N : 0);
+}
+
+// The fused potential over N flat trials: D datasets of T trials each (trial_offsets == null, N = D * T), or D
+// ragged sessions, session d owning flat trials [trial_offsets[d], trial_offsets[d + 1]) (T unused).
+static int tc_loglik_sum(const char *entry, void *handle, const float *theta_dev, int64_t ld_theta, const float *x_dev,
+                         const float *pulses_dev, int64_t ld_pulses, const int64_t *trial_offsets_dev, int64_t D, int64_t T,
+                         int64_t N, int64_t C, float *out_dev, float *workspace_dev, void *stream)
+{
+    Handle *H = live_handle(handle, entry, true);
+    if (H == nullptr) return DDM_ERR_STATE;
+    DDM_REQUIRE(D >= 0 && T >= 0 && N >= 0 && C >= 0 && D <= 0x7FFFFFFFll && T <= 0x7FFFFFFFll && C <= 0x7FFFFFFFll - kTcM,
+                "%s: D=%lld T=%lld N=%lld C=%lld out of range", entry, (long long)D, (long long)T, (long long)N, (long long)C);
+    if (C == 0 || D == 0) return DDM_OK;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    DDM_REQUIRE(out_dev != nullptr, "%s: null output", entry);
+    if (N == 0) {
+        DDM_CUDA_TRY(cudaMemsetAsync(out_dev, 0, (size_t)D * (size_t)C * sizeof(float), st));
+        return DDM_OK;
+    }
+    DDM_REQUIRE(theta_dev && x_dev && pulses_dev && workspace_dev, "%s: null pointer", entry);
+    DDM_REQUIRE(ld_theta >= 5 && ld_pulses >= kCond - 5, "%s: ld_theta=%lld ld_pulses=%lld too small", entry,
+                (long long)ld_theta, (long long)ld_pulses);
+    DDM_REQUIRE((reinterpret_cast<uintptr_t>(workspace_dev) & 15u) == 0, "%s: workspace must be 16-byte aligned", entry);
+    const long long CB = (C + kTcM - 1) / kTcM;
+    const long long n_tiles = N * CB;
+    DDM_REQUIRE(N <= 0x7FFFFFFFll / kHoistTrials && n_tiles <= 0x7FFFFFFFll && D * CB <= 0x7FFFFFFFll,
+                "%s: N * ceil(C / 128) = %lld tiles is too many", entry, n_tiles);
+    float *hoist, *partial;
+    unsigned int *counters;
+    int *sess;
+    tc_sum_workspace(workspace_dev, D, N, C, trial_offsets_dev != nullptr, &hoist, &partial, &counters, &sess);
+    const long long hoist_blocks = (N + kHoistTrials - 1) / kHoistTrials;
+    DDM_REQUIRE(hoist_blocks <= 65535, "%s: %lld trials is too many for one call", entry, (long long)N);
+    const long long *offsets = reinterpret_cast<const long long *>(trial_offsets_dev);
+    auto hoist_kernel = offsets != nullptr ? mnle_hoist_kernel<true> : mnle_hoist_kernel<false>;
+    hoist_kernel<<<dim3(kNets, (unsigned)hoist_blocks), kHidden, 0, st>>>(H->params, H->layout, x_dev, pulses_dev, ld_pulses, (int)N,
+                                                                       hoist, counters, (int)(D * CB), offsets, (int)D, (int)C, sess,
+                                                                       out_dev);
+    DDM_CUDA_TRY(cudaGetLastError());
+    auto kernel = offsets != nullptr ? mnle_tc_kernel<false, false, false, false, true> : mnle_tc_kernel<false>;
+    DDM_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcSmem<false>::kBytes));
+    int sms = 0, n_pairs = 0;
+    long long grid = 0;
+    DDM_CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, H->device));
+    tc_grid(n_tiles, sms, &n_pairs, &grid);
+    kernel<<<(unsigned)grid, kTcThreads, TcSmem<false>::kBytes, st>>>(
+        static_cast<const unsigned char *>(H->tc_pack), H->tc_plan, theta_dev, ld_theta, x_dev, hoist, (int)D, (int)T, (int)C,
+        n_pairs, H->mu_y, H->sigma_y, H->layout.n_choices, partial, counters, out_dev, g_tc_trace, nullptr, TcTrainDump{}, sess,
+        offsets);
+    DDM_CUDA_TRY(cudaGetLastError());
+    return DDM_OK;
+}
+
 DDM_API size_t mnle_loglik_batched_tc_workspace_floats(int64_t D, int64_t T, int64_t C)
 {
     if (D <= 0 || T <= 0 || C <= 0) return 0;
-    return (size_t)D * T * kNets * kHidden + (size_t)D * T * (size_t)C + (size_t)D * (size_t)((C + kTcM - 1) / kTcM);
+    return tc_sum_workspace(nullptr, D, D * T, C, false, nullptr, nullptr, nullptr, nullptr);
 }
 
 DDM_API size_t mnle_loglik_tc_workspace_floats(int64_t T, int64_t C)
@@ -1228,47 +1314,19 @@ DDM_API size_t mnle_loglik_tc_workspace_floats(int64_t T, int64_t C)
     return mnle_loglik_batched_tc_workspace_floats(1, T, C);
 }
 
+DDM_API size_t mnle_loglik_sessions_tc_workspace_floats(int64_t D, int64_t N, int64_t C)
+{
+    if (D <= 0 || N <= 0 || C <= 0) return 0;
+    return tc_sum_workspace(nullptr, D, N, C, true, nullptr, nullptr, nullptr, nullptr);
+}
+
 DDM_API int mnle_loglik_sum_batched_tc_f32(void *handle, const float *theta_dev, int64_t ld_theta, const float *x_dev,
                                            const float *pulses_dev, int64_t ld_pulses, int64_t D, int64_t T, int64_t C,
                                            float *out_dev, float *workspace_dev, void *stream)
 {
-    Handle *H = live_handle(handle, "mnle_loglik_sum_tc", true);
-    if (H == nullptr) return DDM_ERR_STATE;
-    DDM_REQUIRE(D >= 0 && T >= 0 && C >= 0 && D <= 0x7FFFFFFFll && T <= 0x7FFFFFFFll && C <= 0x7FFFFFFFll - kTcM,
-                "mnle_loglik_sum_tc: D=%lld T=%lld C=%lld out of range", (long long)D, (long long)T, (long long)C);
-    if (C == 0 || D == 0) return DDM_OK;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    DDM_REQUIRE(out_dev != nullptr, "mnle_loglik_sum_tc: null output");
-    if (T == 0) {
-        DDM_CUDA_TRY(cudaMemsetAsync(out_dev, 0, (size_t)D * (size_t)C * sizeof(float), st));
-        return DDM_OK;
-    }
-    DDM_REQUIRE(theta_dev && x_dev && pulses_dev && workspace_dev, "mnle_loglik_sum_tc: null pointer");
-    DDM_REQUIRE(ld_theta >= 5 && ld_pulses >= kCond - 5, "mnle_loglik_sum_tc: ld_theta=%lld ld_pulses=%lld too small",
-                (long long)ld_theta, (long long)ld_pulses);
-    DDM_REQUIRE((reinterpret_cast<uintptr_t>(workspace_dev) & 15u) == 0, "mnle_loglik_sum_tc: workspace must be 16-byte aligned");
-    const long long CB = (C + kTcM - 1) / kTcM;
-    const long long n_tiles = D * T * CB;
-    DDM_REQUIRE(D * T <= 0x7FFFFFFFll / kHoistTrials && n_tiles <= 0x7FFFFFFFll && D * CB <= 0x7FFFFFFFll,
-                "mnle_loglik_sum_tc: D * T * ceil(C / 128) = %lld tiles is too many", n_tiles);
-    float *hoist = workspace_dev;
-    float *partial = hoist + (size_t)D * T * kNets * kHidden;
-    unsigned int *counters = reinterpret_cast<unsigned int *>(partial + (size_t)D * T * (size_t)C);
-    const long long hoist_blocks = (D * T + kHoistTrials - 1) / kHoistTrials;
-    DDM_REQUIRE(hoist_blocks <= 65535, "mnle_loglik_sum_tc: D * T = %lld trials is too many for one call", (long long)(D * T));
-    mnle_hoist_kernel<<<dim3(kNets, (unsigned)hoist_blocks), kHidden, 0, st>>>(H->params, H->layout, x_dev, pulses_dev, ld_pulses,
-                                                                            (int)(D * T), hoist, counters, (int)(D * CB));
-    DDM_CUDA_TRY(cudaGetLastError());
-    DDM_CUDA_TRY(cudaFuncSetAttribute(mnle_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcSmem<false>::kBytes));
-    int sms = 0, n_pairs = 0;
-    long long grid = 0;
-    DDM_CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, H->device));
-    tc_grid(n_tiles, sms, &n_pairs, &grid);
-    mnle_tc_kernel<false><<<(unsigned)grid, kTcThreads, TcSmem<false>::kBytes, st>>>(
-        static_cast<const unsigned char *>(H->tc_pack), H->tc_plan, theta_dev, ld_theta, x_dev, hoist, (int)D, (int)T, (int)C,
-        n_pairs, H->mu_y, H->sigma_y, H->layout.n_choices, partial, counters, out_dev, g_tc_trace);
-    DDM_CUDA_TRY(cudaGetLastError());
-    return DDM_OK;
+    const bool in_range = D >= 0 && T >= 0 && D <= 0x7FFFFFFFll && T <= 0x7FFFFFFFll;   // (N = -1 is reported as out of range)
+    return tc_loglik_sum("mnle_loglik_sum_tc", handle, theta_dev, ld_theta, x_dev, pulses_dev, ld_pulses, nullptr, D, T,
+                         in_range ? D * T : -1, C, out_dev, workspace_dev, stream);
 }
 
 DDM_API int mnle_loglik_sum_tc_f32(void *handle, const float *theta_dev, int64_t ld_theta, const float *x_dev,
@@ -1277,6 +1335,15 @@ DDM_API int mnle_loglik_sum_tc_f32(void *handle, const float *theta_dev, int64_t
 {
     return mnle_loglik_sum_batched_tc_f32(handle, theta_dev, ld_theta, x_dev, pulses_dev, ld_pulses, 1, T, C, out_dev,
                                           workspace_dev, stream);
+}
+
+DDM_API int mnle_loglik_sum_sessions_tc_f32(void *handle, const float *theta_dev, int64_t ld_theta, const float *x_dev,
+                                            const float *pulses_dev, int64_t ld_pulses, const int64_t *trial_offsets_dev,
+                                            int64_t D, int64_t N, int64_t C, float *out_dev, float *workspace_dev, void *stream)
+{
+    DDM_REQUIRE(trial_offsets_dev != nullptr || D == 0, "mnle_loglik_sum_sessions_tc_f32: null trial_offsets");
+    return tc_loglik_sum("mnle_loglik_sum_sessions_tc_f32", handle, theta_dev, ld_theta, x_dev, pulses_dev, ld_pulses,
+                         trial_offsets_dev, D, 0, N, C, out_dev, workspace_dev, stream);
 }
 
 DDM_API int mnle_log_prob_rows_tc_f32(void *handle, const float *x_dev, const float *cond_dev, int64_t ld_cond, int64_t R,

@@ -907,17 +907,25 @@ DDM_API int mnle_train_adam_f32(float *params_dev, const float *grad_dev, float 
 // columns of every first layer are contracted: grad[c][i] = sum_t sum_net sum_j DH[net][0][j][t*C+c] W1_net[j][i].
 namespace mnle {
 
+// Ragged sessions (offsets != null, D + 1 entries): t is the flat trial, and its rows take the chains of its session,
+// theta row session_of(t) * C + c.
 __global__ void __launch_bounds__(256) potential_rows_kernel(const float *__restrict__ theta, long long ld_theta,
                                                              const float *__restrict__ x, const float *__restrict__ pulses,
                                                              long long ld_pulses, int T, int C, float *__restrict__ cond,
-                                                             float *__restrict__ xr)
+                                                             float *__restrict__ xr, const long long *__restrict__ offsets = nullptr,
+                                                             int D = 1)
 {
     const long long total = (long long)T * C * kCond;
     for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long long)gridDim.x * blockDim.x) {
         const long long r = idx / kCond;
         const int j = (int)(idx - r * kCond);
         const int t = (int)(r / C), c = (int)(r - (long long)t * C);
-        cond[idx] = j < 5 ? __ldg(theta + (long long)c * ld_theta + j) : __ldg(pulses + (long long)t * ld_pulses + (j - 5));
+        if (j < 5) {
+            const long long th_row = offsets != nullptr ? (long long)session_of(offsets, D, t) * C + c : c;
+            cond[idx] = __ldg(theta + th_row * ld_theta + j);
+        } else {
+            cond[idx] = __ldg(pulses + (long long)t * ld_pulses + (j - 5));
+        }
         if (j < 2) xr[2 * r + j] = __ldg(x + 2 * t + j);
     }
 }
@@ -997,13 +1005,13 @@ static PotentialGradBufs potential_grad_workspace(Carver &ws, const Layout &L, c
     return b;
 }
 
-// The argument checks and empty cases of the two potentials over expanded (trial, chain) rows.  *H is set when there
+// The argument checks and empty cases of the potentials over expanded (trial, chain) rows.  *H is set when there
 // are rows to evaluate; otherwise the return value is final: an error, or DDM_OK when C == 0, or when T == 0 once out_dev
-// and (want_grad) grad_dev are zeroed.
+// (n_sets * C: one sum per dataset and chain) and (want_grad) grad_dev are zeroed.
 static int expanded_rows_prologue(const char *entry, Handle **H, void *handle, const float *theta_dev, int64_t ld_theta,
                                   const float *x_dev, const float *pulses_dev, int64_t ld_pulses, int64_t T, int64_t C,
                                   float *out_dev, bool want_grad, float *grad_dev, const float *workspace_dev,
-                                  cudaStream_t st)
+                                  cudaStream_t st, int64_t n_sets = 1)
 {
     *H = nullptr;
     Handle *h = live_handle(handle, entry);
@@ -1013,7 +1021,7 @@ static int expanded_rows_prologue(const char *entry, Handle **H, void *handle, c
     if (C == 0) return DDM_OK;
     DDM_REQUIRE(out_dev && (grad_dev || !want_grad), "%s: null output", entry);
     if (T == 0) {
-        DDM_CUDA_TRY(cudaMemsetAsync(out_dev, 0, (size_t)C * sizeof(float), st));
+        DDM_CUDA_TRY(cudaMemsetAsync(out_dev, 0, (size_t)n_sets * (size_t)C * sizeof(float), st));
         if (want_grad) DDM_CUDA_TRY(cudaMemsetAsync(grad_dev, 0, (size_t)C * 5 * sizeof(float), st));
         return DDM_OK;
     }
@@ -1209,13 +1217,19 @@ __global__ void __launch_bounds__(kRowWarps * 32) precise_rows_kernel(const floa
     }
 }
 
-__global__ void __launch_bounds__(128) precise_sum_kernel(const double *__restrict__ LP, int T, int C, float *__restrict__ out)
+// grid (chain blocks of 128, D): out[d * C + c] = the fp64 sum over the T_d trials of dataset d, in trial order.  One
+// dataset of T trials (offsets == null, D = 1), or ragged sessions, session d owning trials [offsets[d], offsets[d + 1]).
+__global__ void __launch_bounds__(128) precise_sum_kernel(const double *__restrict__ LP, const long long *__restrict__ offsets,
+                                                          int T, int C, float *__restrict__ out)
 {
-    const int c = blockIdx.x * 128 + threadIdx.x;
+    const int c = blockIdx.x * 128 + threadIdx.x, d = blockIdx.y;
     if (c >= C) return;
+    const long long first = offsets != nullptr ? offsets[d] : 0;
+    const int Td = offsets != nullptr ? (int)(offsets[d + 1] - first) : T;
+    const double *col = LP + (size_t)first * C + c;
     double sum = 0.0;
-    for (int t = 0; t < T; ++t) sum += LP[(size_t)t * C + c];
-    out[c] = (float)sum;
+    for (int t = 0; t < Td; ++t) sum += col[(size_t)t * C];
+    out[(size_t)d * C + c] = (float)sum;
 }
 
 struct Tc64Bufs {
@@ -1250,22 +1264,25 @@ DDM_API size_t mnle_loglik_tc64_workspace_floats(int n_choices, int64_t T, int64
     return ws.floats();
 }
 
-DDM_API int mnle_loglik_sum_tc64_f32(void *handle, const float *theta_dev, int64_t ld_theta, const float *x_dev,
-                                     const float *pulses_dev, int64_t ld_pulses, int64_t T, int64_t C, float *out_dev,
-                                     float *workspace_dev, void *stream)
+namespace mnle {
+
+// tc64 over N flat trials: one dataset (trial_offsets == null, N = T) or D ragged sessions (see precise_sum_kernel).
+static int tc64_loglik_sum(const char *entry, void *handle, const float *theta_dev, int64_t ld_theta, const float *x_dev,
+                           const float *pulses_dev, int64_t ld_pulses, const int64_t *trial_offsets_dev, int64_t D, int64_t N,
+                           int64_t C, float *out_dev, float *workspace_dev, cudaStream_t st)
 {
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
     Handle *H;
-    int rc = expanded_rows_prologue("mnle_loglik_sum_tc64_f32", &H, handle, theta_dev, ld_theta, x_dev, pulses_dev, ld_pulses, T,
-                                    C, out_dev, false, nullptr, workspace_dev, st);
+    int rc = expanded_rows_prologue(entry, &H, handle, theta_dev, ld_theta, x_dev, pulses_dev, ld_pulses, N, C, out_dev, false,
+                                    nullptr, workspace_dev, st, D);
     if (H == nullptr) return rc;
     const Layout &L = H->layout;
-    const long long R = T * C;
+    const long long R = N * C;
     const TrainDims d = train_dims(L, R);
     Carver ws(workspace_dev);
     const Tc64Bufs B = tc64_workspace(ws, L, d);
+    const long long *offsets = reinterpret_cast<const long long *>(trial_offsets_dev);
     potential_rows_kernel<<<(unsigned)std::min<long long>((R * kCond + 255) / 256, 148 * 16), 256, 0, st>>>(
-        theta_dev, ld_theta, x_dev, pulses_dev, ld_pulses, (int)T, (int)C, B.cond, B.xr);
+        theta_dev, ld_theta, x_dev, pulses_dev, ld_pulses, (int)N, (int)C, B.cond, B.xr, offsets, (int)D);
     DDM_CUDA_TRY(cudaGetLastError());
     const TcTrainDump keep{nullptr, B.Q, B.LG, d.Rp, nullptr, nullptr, nullptr};
     rc = tc_train_forward(H->params, L, B.pack, B.xr, B.cond, (long long)kCond, nullptr, R, keep, B.lp32, st);
@@ -1273,9 +1290,35 @@ DDM_API int mnle_loglik_sum_tc64_f32(void *handle, const float *theta_dev, int64
     precise_rows_kernel<<<(unsigned)((R + kBlockRows - 1) / kBlockRows), kRowWarps * 32, 0, st>>>(B.Q, B.LG, d.Rp, B.xr, R, L.n_choices,
                                                                                                   H->mu_y, H->sigma_y, B.LP);
     DDM_CUDA_TRY(cudaGetLastError());
-    precise_sum_kernel<<<(unsigned)((C + 127) / 128), 128, 0, st>>>(B.LP, (int)T, (int)C, out_dev);
+    precise_sum_kernel<<<dim3((unsigned)((C + 127) / 128), (unsigned)D), 128, 0, st>>>(B.LP, offsets, (int)N, (int)C, out_dev);
     DDM_CUDA_TRY(cudaGetLastError());
     return DDM_OK;
+}
+
+}  // namespace mnle
+
+DDM_API int mnle_loglik_sum_tc64_f32(void *handle, const float *theta_dev, int64_t ld_theta, const float *x_dev,
+                                     const float *pulses_dev, int64_t ld_pulses, int64_t T, int64_t C, float *out_dev,
+                                     float *workspace_dev, void *stream)
+{
+    return tc64_loglik_sum("mnle_loglik_sum_tc64_f32", handle, theta_dev, ld_theta, x_dev, pulses_dev, ld_pulses, nullptr, 1, T,
+                           C, out_dev, workspace_dev, static_cast<cudaStream_t>(stream));
+}
+
+DDM_API size_t mnle_loglik_sessions_tc64_workspace_floats(int n_choices, int64_t D, int64_t N, int64_t C)
+{
+    return D <= 0 ? 0 : mnle_loglik_tc64_workspace_floats(n_choices, N, C);
+}
+
+DDM_API int mnle_loglik_sum_sessions_tc64_f32(void *handle, const float *theta_dev, int64_t ld_theta, const float *x_dev,
+                                              const float *pulses_dev, int64_t ld_pulses, const int64_t *trial_offsets_dev,
+                                              int64_t D, int64_t N, int64_t C, float *out_dev, float *workspace_dev, void *stream)
+{
+    DDM_REQUIRE(D >= 0 && D <= 65535, "mnle_loglik_sum_sessions_tc64_f32: D=%lld sessions (at most 65535 per call)", (long long)D);
+    if (D == 0) return DDM_OK;
+    DDM_REQUIRE(trial_offsets_dev != nullptr, "mnle_loglik_sum_sessions_tc64_f32: null trial_offsets");
+    return tc64_loglik_sum("mnle_loglik_sum_sessions_tc64_f32", handle, theta_dev, ld_theta, x_dev, pulses_dev, ld_pulses,
+                           trial_offsets_dev, D, N, C, out_dev, workspace_dev, static_cast<cudaStream_t>(stream));
 }
 
 // ---- estimator.sample: the choice from the categorical net, then log rt from the flow run in inverse --------------

@@ -71,16 +71,39 @@ def run_inference_mcmc(cfg, prior_theta, density_estimator, x_o, pulses_o, *, nu
 
 
 class _BatchedPotential:
-    """log prior + loglik / temperature for D datasets x C chains as one flat (D*C, 5) batch."""
+    """log prior + loglik / temperature for D datasets x C chains as one flat (D*C, 5) batch: datasets of equal
+    length (x (D,T,2), pulses (D,T,>=80)), or with ``plan`` (a ``SessionPlan``) ragged sessions one after the other
+    (x (N,2), pulses (N,>=80))."""
 
-    def __init__(self, estimator, prior_theta, x, pulses, temperature: float):
-        self.est, self.prior, self.x, self.pulses = estimator, prior_theta, x, pulses
-        self.D, self.temperature = x.shape[0], float(temperature)
+    def __init__(self, estimator, prior_theta, x, pulses, temperature: float, plan=None):
+        self.est, self.prior, self.x, self.pulses, self.plan = estimator, prior_theta, x, pulses, plan
+        self.D, self.temperature = (x.shape[0] if plan is None else plan.D), float(temperature)
 
     def __call__(self, theta_flat: torch.Tensor) -> torch.Tensor:
         lp = prior_log_prob(self.prior, theta_flat)
-        ll = self.est.loglik_sum_batched(theta_flat.view(self.D, -1, theta_flat.shape[-1]), self.x, self.pulses).reshape(-1)
-        return torch.where(torch.isfinite(lp), lp + ll / self.temperature, lp)
+        th = theta_flat.view(self.D, -1, theta_flat.shape[-1])
+        if self.plan is None:
+            ll = self.est.loglik_sum_batched(th, self.x, self.pulses)
+        else:
+            ll = self.est.loglik_sum_sessions(th, self.x, self.pulses, self.plan, kernel=self.plan.kernel)
+        return torch.where(torch.isfinite(lp), lp + ll.reshape(-1) / self.temperature, lp)
+
+
+def _sample_groups(cfg, potential, init: torch.Tensor, G: int, first: int, num_samples: int, seed: int, what: str
+                   ) -> torch.Tensor:
+    """The sampling core of ``sbc_shard`` and ``sessions_shard``: G groups (datasets / sessions, global numbers
+    first .. first + G - 1) of C chains each, all in lock-step through one potential call per iteration, each group
+    with its own slice widths and every chain with its own counter-based uniforms (Philox rows of the GLOBAL chain
+    numbers).  -> (G, num_samples, 5) CPU."""
+    S, C = int(num_samples), init.shape[0] // G
+    ok = torch.isfinite(potential(init)).view(G, C).all(dim=1)
+    if not bool(ok.all()):
+        raise RuntimeError(f"a prior draw of {what} {first + int((~ok).nonzero()[0])} has a non-finite posterior potential")
+    sampler = VectorizedSliceSampler(GraphedLogProb(potential, init), init, chain_groups=G,
+                                     uniforms=PhiloxUniforms(int(seed) * 1_000_003 + 17, first * C, G * C, init.device))
+    per_chain = -(-S // C)
+    draws = sampler.run(per_chain, warmup=int(cfg.WARMUP_STEPS), thin=1)                  # (per_chain, G*C, 5)
+    return draws.view(per_chain, G, C, 5).permute(1, 0, 2, 3).reshape(G, per_chain * C, 5)[:, :S].cpu()
 
 
 @torch.no_grad()
@@ -105,13 +128,7 @@ def sbc_shard(cfg, prior_theta, estimator, thetas_true: torch.Tensor, ds_seeds, 
         x[..., 0] = torch.log(x[..., 0].clamp_min(1e-6))
     potential = _BatchedPotential(estimator, prior_theta, x, pulses, float(cfg.TEMPERATURE))
     init = init_all[lo * C:hi * C].to(device=dev, dtype=torch.float32)
-    if not bool(torch.isfinite(potential(init)).all()):
-        raise RuntimeError("a prior draw has a non-finite posterior potential")
-    sampler = VectorizedSliceSampler(GraphedLogProb(potential, init), init, chain_groups=D,
-                                     uniforms=PhiloxUniforms(int(seed) * 1_000_003 + 17, lo * C, D * C, dev))
-    per_chain = -(-S // C)
-    draws = sampler.run(per_chain, warmup=int(cfg.WARMUP_STEPS), thin=1)                  # (per_chain, D*C, 5)
-    samples = draws.view(per_chain, D, C, 5).permute(1, 0, 2, 3).reshape(D, per_chain * C, 5)[:, :S].cpu()
+    samples = _sample_groups(cfg, potential, init, D, lo, S, seed, "dataset")
     for i in range(D):
         ranks[i] = compute_ranks(thetas_true[lo + i], samples[i])
     return ranks, samples
@@ -146,6 +163,72 @@ def run_sbc(cfg, *, prior_theta, density_estimator, device: str = "cpu", num_dat
         np.save(os.path.join(outdir, "sbc_thetas_true.npy"), out["thetas_true"])
         np.save(os.path.join(outdir, "sbc_ranks.npy"), out["ranks"])   # (the reference also draws a histogram: not on this path)
     return out
+
+
+def _session_tensors(sessions, first: int, dev):
+    """(x (T_i,2), pulses (T_i,80)) fp32 on ``dev`` of every session, checked on the host."""
+    xs, pls = [], []
+    for i, (x, pl) in enumerate(sessions):
+        x = x.to(device=dev, dtype=torch.float32)
+        if x.dim() == 3 and x.shape[1] == 1:
+            x = x[:, 0, :]
+        if x.dim() != 2 or x.shape[1] != 2:
+            raise ValueError(f"session {first + i}: x_o must be (T,2), got {tuple(x.shape)}")
+        if pl.dim() != 2 or pl.shape[0] != x.shape[0] or pl.shape[1] < 80:
+            raise ValueError(f"session {first + i}: pulses must be (T,>=80) with T={x.shape[0]}, got {tuple(pl.shape)}")
+        xs.append(x)
+        pls.append(pl[:, :80].to(device=dev, dtype=torch.float32))
+    return xs, pls
+
+
+@torch.no_grad()
+def sessions_shard(cfg, prior_theta, estimator, sessions, init_all: torch.Tensor, lo: int, hi: int, seed: int,
+                   kernel: str = "tc", device=None) -> torch.Tensor:
+    """Sessions [lo, hi) of ``run_inference_sessions``: all their chains sampled in lock-step through one ragged
+    potential call per iteration (the counterpart of ``sbc_shard``, same sampling core).  ``init_all``: the starting
+    points of ALL sessions, C per session.  -> (hi-lo, cfg.POSTERIOR_SAMPLES, 5) float32 CPU.  Everything random is
+    indexed by the global session / chain number, so any split into shards reproduces the unsplit run bit for bit."""
+    dev = compute_device(device)
+    G, S = hi - lo, int(cfg.POSTERIOR_SAMPLES)
+    if G == 0:
+        return torch.empty((0, S, 5), dtype=torch.float32)
+    C = init_all.shape[0] // len(sessions)
+    xs, pls = _session_tensors(sessions[lo:hi], lo, dev)
+    est = as_device_estimator(estimator)
+    plan = est.session_plan([x.shape[0] for x in xs], C, kernel=kernel, device=dev)
+    potential = _BatchedPotential(est, prior_theta, torch.cat(xs), torch.cat(pls), float(cfg.TEMPERATURE), plan=plan)
+    init = init_all[lo * C:hi * C].to(device=dev, dtype=torch.float32)
+    return _sample_groups(cfg, potential, init, G, lo, S, seed, "session")
+
+
+@torch.no_grad()
+def run_inference_sessions(cfg, prior_theta, density_estimator, sessions, *, num_chains: Optional[int] = None, seed: int = 0,
+                           kernel: str = "tc", device=None, group=None) -> list:
+    """Posterior samples over theta (dim 5) for each of several observed sessions of any lengths, from one estimator
+    in one run: ``sessions`` is a sequence of (x_o (T_i,2), pulses_o (T_i,>=80)); x_o is used as given, as
+    ``run_inference_mcmc`` uses it.  Returns one (cfg.POSTERIOR_SAMPLES, 5) float32 CPU tensor per session.
+
+    ``num_chains`` per session defaults to max(cfg.NUM_CHAINS, 128); cfg.WARMUP_STEPS tuning sweeps and
+    cfg.TEMPERATURE as in ``run_inference_mcmc``.  ``kernel``: "tc" or "tc64" (``DeviceMNLE.loglik_sum_sessions``).
+    The starting points are prior draws under ``torch.manual_seed(seed)`` in a forked RNG state (the caller's stream
+    is left alone), the sampler's uniforms are keyed by ``seed`` and the global chain number.  Under torchrun the
+    sessions are split over the ranks (``shard_bounds``) and the draws all-gathered: every rank returns the full
+    list, identical for any world size."""
+    sessions = list(sessions)
+    n = len(sessions)
+    if n == 0:
+        return []
+    dev = compute_device(device)
+    C = int(num_chains) if num_chains is not None else max(int(cfg.NUM_CHAINS), MIN_VECTOR_CHAINS)
+    cuda_devices = list(range(torch.cuda.device_count())) if torch.cuda.is_initialized() else []
+    with torch.random.fork_rng(devices=cuda_devices):
+        torch.manual_seed(int(seed))
+        init_all = prior_theta.sample((n * C,)).to(torch.float32)
+    rank, world = _world(group)
+    lo, hi = shard_bounds(n, rank, world)
+    local = sessions_shard(cfg, prior_theta, density_estimator, sessions, init_all, lo, hi, seed, kernel, dev)
+    samples = all_gather_rows(local.to(dev), n, group).cpu()
+    return [samples[i] for i in range(n)]
 
 
 # ---- checkpoints (reference mnle.py:241-297) ---------------------------------------------------------------

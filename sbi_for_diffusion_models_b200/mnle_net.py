@@ -48,6 +48,61 @@ def unpack_params(packed: torch.Tensor, n_choices: int) -> Dict[str, torch.Tenso
     return out
 
 
+def session_offsets(lengths) -> np.ndarray:
+    """Trial offsets (D+1,) int64 of ragged sessions: session d owns flat trials [offsets[d], offsets[d+1]).
+    ``lengths``: a sequence or 1-D CPU integer tensor of D non-negative session lengths."""
+    if isinstance(lengths, torch.Tensor):
+        if lengths.device.type != "cpu" or lengths.ndim != 1 or lengths.is_floating_point() or lengths.is_complex():
+            raise ValueError(f"lengths must be a 1-D CPU integer tensor, got {lengths.dtype} {tuple(lengths.shape)} "
+                             f"on {lengths.device}")
+        arr = lengths.to(torch.int64).numpy()
+    else:
+        arr = np.asarray(list(lengths))
+        if arr.size == 0:
+            arr = arr.astype(np.int64)
+        if arr.ndim != 1 or not np.issubdtype(arr.dtype, np.integer):
+            raise ValueError(f"lengths must be a sequence of ints, got {arr.dtype} {arr.shape}")
+    arr = arr.astype(np.int64)
+    if arr.size and int(arr.min()) < 0:
+        raise ValueError(f"session lengths must be non-negative, got {int(arr.min())} for session {int(arr.argmin())}")
+    return np.concatenate([np.zeros(1, np.int64), np.cumsum(arr)])
+
+
+def split_sessions(offsets: np.ndarray, max_trials: int, max_sessions: int) -> list:
+    """Consecutive session ranges [d0, d1) covering all D sessions, each with at most ``max_trials`` trials and
+    ``max_sessions`` sessions: the launches of one ragged potential call.  A single session longer than
+    ``max_trials`` raises ValueError."""
+    D = len(offsets) - 1
+    chunks, d0 = [], 0
+    for d in range(D):
+        if offsets[d + 1] - offsets[d] > max_trials:
+            raise ValueError(f"session {d} has {int(offsets[d + 1] - offsets[d])} trials, more than the {max_trials} "
+                             "one launch can take")
+        if d > d0 and (offsets[d + 1] - offsets[d0] > max_trials or d - d0 >= max_sessions):
+            chunks.append((d0, d))
+            d0 = d
+    if D:
+        chunks.append((d0, D))
+    return chunks
+
+
+class SessionPlan:
+    """D ragged sessions laid out for ``DeviceMNLE.loglik_sum_sessions`` with C chains each and one kernel: the trial
+    offsets (checked on the host), their split into launches at session boundaries, and each launch's offsets on the
+    device.  Built once (``DeviceMNLE.session_plan``); a call through it copies nothing between host and device, so
+    a CUDA graph can record it."""
+
+    def __init__(self, lengths, C: int, kernel: str, device: torch.device, max_trials: int, max_sessions: int):
+        self.offsets = session_offsets(lengths)
+        self.lengths = np.diff(self.offsets)
+        self.D, self.N, self.C, self.kernel, self.device = len(self.offsets) - 1, int(self.offsets[-1]), int(C), kernel, device
+        self.chunks = []
+        for d0, d1 in split_sessions(self.offsets, max_trials, max_sessions):
+            n0, n1 = int(self.offsets[d0]), int(self.offsets[d1])
+            off = torch.from_numpy(self.offsets[d0:d1 + 1] - n0).to(device)
+            self.chunks.append((d0, d1, n0, n1, off))
+
+
 class PackedMNLE:
     """CPU-resident packed parameters + lazily created device handles."""
 
@@ -437,6 +492,68 @@ class DeviceMNLE(torch.nn.Module):
                                                   pl.shape[2], D, T, C, out.data_ptr(), ws.data_ptr(),
                                                   torch.cuda.current_stream(dev).cuda_stream)
             _native.check(rc, "mnle_loglik_sum_batched_tc_f32")
+        return out.to(theta.device)
+
+    SESSIONS_MAX_TRIALS = 524_280        # trials of one mnle_loglik_sum_sessions_tc_f32 launch (its hoist grid)
+    SESSIONS_TC64_MAX_ROWS = 8_000_000   # (trial, chain) rows of one mnle_loglik_sum_sessions_tc64_f32 launch
+    SESSIONS_TC64_MAX_SESSIONS = 65_535  # sessions of one tc64 launch (its final sum's grid)
+
+    def session_plan(self, lengths, C: int, *, kernel: str = "tc", device=None) -> SessionPlan:
+        """The layout ``loglik_sum_sessions`` needs for sessions of these lengths with C chains each, built once: pass
+        it as ``lengths`` to calls that must not touch the host (a sampler's CUDA graph)."""
+        if kernel not in ("tc", "tc64"):
+            raise ValueError(f"unknown kernel {kernel!r} for sessions (tc or tc64)")
+        if kernel == "tc":
+            max_trials, max_sessions = self.SESSIONS_MAX_TRIALS, 2**31 - 1
+        else:
+            max_trials, max_sessions = self.SESSIONS_TC64_MAX_ROWS // max(int(C), 1), self.SESSIONS_TC64_MAX_SESSIONS
+        return SessionPlan(lengths, C, kernel, self._dev() if device is None else torch.device(device), max_trials, max_sessions)
+
+    def loglik_sum_sessions(self, theta: torch.Tensor, x_o: torch.Tensor, pulses: torch.Tensor, lengths, *,
+                            kernel: str = "tc") -> torch.Tensor:
+        """D observed sessions of different lengths in one call: theta (D,C,5), x_o (N,2), pulses (N,>=80) with the
+        sessions' trials one after the other, ``lengths`` the D session lengths (sequence or CPU tensor, sum N) or a
+        ``SessionPlan`` of them -> (D,C), out[d,c] = sum over session d's trials t of log p(x_o[t] | [theta[d,c],
+        pulses[t]]), 0 for an empty session.  Each output has the bits of ``loglik_sum(theta[d], x_d, pulses_d,
+        kernel=kernel)``.  ``kernel``: "tc" (tcgen05) or "tc64" (tensor-core networks, fp64 spline chain).  Requests
+        over one launch's limit are split at session boundaries; shapes and lengths are checked before any launch."""
+        if kernel not in ("tc", "tc64"):
+            raise ValueError(f"unknown kernel {kernel!r} for sessions (tc or tc64)")
+        if theta.ndim != 3 or theta.shape[2] != 5:
+            raise ValueError(f"theta must be (D,C,5), got {tuple(theta.shape)}")
+        D, C = theta.shape[0], theta.shape[1]
+        dev = self._dev(theta)
+        plan = lengths if isinstance(lengths, SessionPlan) else self.session_plan(lengths, C, kernel=kernel, device=dev)
+        if (plan.D, plan.C, plan.kernel, plan.device) != (D, C, kernel, dev):
+            raise ValueError(f"the session plan is for D={plan.D}, C={plan.C}, kernel {plan.kernel!r} on {plan.device}; "
+                             f"the call has D={D}, C={C}, kernel {kernel!r} on {dev}")
+        if x_o.ndim != 2 or tuple(x_o.shape) != (plan.N, 2):
+            raise ValueError(f"x_o must be (N,2) with N={plan.N} (the sum of the lengths), got {tuple(x_o.shape)}")
+        if pulses.ndim != 2 or pulses.shape[0] != plan.N or pulses.shape[1] < COND_DIM - 5:
+            raise ValueError(f"pulses must be (N,>=80) with N={plan.N}, got {tuple(pulses.shape)}")
+        th = theta.to(device=dev, dtype=torch.float32).contiguous()
+        xo = x_o.to(device=dev, dtype=torch.float32).contiguous()
+        pl = pulses.to(device=dev, dtype=torch.float32)
+        if pl.stride(1) != 1 or (pl.shape[0] > 1 and pl.stride(0) < COND_DIM - 5):
+            pl = pl.contiguous()
+        ld_pulses = pl.stride(0) if pl.shape[0] > 1 else pl.shape[1]
+        out = torch.empty((D, C), dtype=torch.float32, device=dev)
+        if D == 0 or C == 0:
+            return out.to(theta.device)
+        L = _native.lib()
+        if kernel == "tc":
+            fn, ws_floats = L.mnle_loglik_sum_sessions_tc_f32, L.mnle_loglik_sessions_tc_workspace_floats
+        else:
+            fn = L.mnle_loglik_sum_sessions_tc64_f32
+            ws_floats = lambda d, n, c: L.mnle_loglik_sessions_tc64_workspace_floats(self.packed.n_choices, d, n, c)
+        with torch.cuda.device(dev):
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            n_ws = max(ws_floats(d1 - d0, n1 - n0, C) for d0, d1, n0, n1, _ in plan.chunks)
+            ws = torch.empty((max(n_ws, 1),), dtype=torch.float32, device=dev)   # torch allocations are 512-byte aligned
+            for d0, d1, n0, n1, off in plan.chunks:
+                rc = fn(self.packed.handle(dev), th[d0].data_ptr(), 5, xo[n0:].data_ptr(), pl[n0:].data_ptr(), ld_pulses,
+                        off.data_ptr(), d1 - d0, n1 - n0, C, out[d0].data_ptr(), ws.data_ptr(), stream)
+                _native.check(rc, "mnle_loglik_sum_sessions")
         return out.to(theta.device)
 
     @staticmethod
