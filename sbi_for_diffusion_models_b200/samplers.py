@@ -91,6 +91,8 @@ class VectorizedSliceSampler:
     potential plus ~60 elementwise ops of bookkeeping) is captured once into a CUDA graph and replayed.
     """
 
+    MAX_FUSED_DIM = 64      # the largest D the kernels of csrc/mnle_sampler.cu accept
+
     def __init__(self, log_prob_fn: Callable[[torch.Tensor], torch.Tensor], init: torch.Tensor, *,
                  init_width: float = 0.1, max_step_out: int = 8, max_shrink: int = 64,
                  generator: Optional[torch.Generator] = None, uniforms: Optional[Callable[[int], torch.Tensor]] = None,
@@ -116,10 +118,13 @@ class VectorizedSliceSampler:
         self.max_step_out, self.max_shrink = int(max_step_out), int(max_shrink)
         self._use_graph = bool(use_graph) and init.is_cuda
         # the bookkeeping of an iteration as two CUDA kernels around the potential (csrc/mnle_sampler.cu) instead of
-        # ~80 elementwise torch launches; same arithmetic in the same order, same bits (float32 chains on a GPU)
-        self._fused = (init.is_cuda and init.dtype == torch.float32) if fused is None else bool(fused)
-        if self._fused and not (init.is_cuda and init.dtype == torch.float32):
-            raise ValueError("the fused sampler kernels need float32 chains on a CUDA device")
+        # ~80 elementwise torch launches; same arithmetic in the same order, same bits (float32 chains on a GPU, at
+        # most MAX_FUSED_DIM coordinates; by default larger D runs the torch implementation, fused=True refuses it)
+        fusable = init.is_cuda and init.dtype == torch.float32 and self.D <= self.MAX_FUSED_DIM
+        self._fused = fusable if fused is None else bool(fused)
+        if self._fused and not fusable:
+            raise ValueError(f"the fused sampler kernels need float32 chains on a CUDA device and at most "
+                             f"{self.MAX_FUSED_DIM} coordinates, got {init.dtype} on {init.device}, D = {self.D}")
         self._graph = None
         self._it = 0
 
@@ -211,7 +216,7 @@ class VectorizedSliceSampler:
         fin = (acc | (give_up & live))
         tune = fin & (self.sweeps < self._warmup)
         cnt = self.tuned[idx, self.d]
-        self.width[idx, self.d] = torch.where(tune, w + ((hi - lo) - w) / (cnt + 1.0), w).clamp_min(1e-6)
+        self.width[idx, self.d] = torch.where(tune, (w + ((hi - lo) - w) / (cnt + 1.0)).clamp_min(1e-6), w)
         self.tuned[idx, self.d] = cnt + tune.to(cnt.dtype)
         sweep_end = fin & (self.d == D - 1)
         self.d.copy_(torch.where(fin, (self.d + 1) % D, self.d))
