@@ -439,6 +439,40 @@ int mnle_tc_set_trace(long long *trace_dev);
 int mnle_tc_selftest(const float *a_dev, const float *b_dev, int N, int passes, uint32_t lbo_a,
                      uint32_t lbo_b, uint32_t sbo, float *d_dev, void *stream);
 
+/* ------------------------------------------------- grid likelihood of the DDM --- */
+
+/*
+ * The simulator's own law, computed instead of sampled: the accumulator's density is propagated on a grid of
+ * M cells over (0, B), one Euler step at a time, and the mass absorbed at each bound on each step is read off
+ * (oracle/ddm_grid_spec.py defines the scheme in float64).  M = clamp(ceil(B * cells_per_sigma / noise_scale), 1,
+ * ddm_grid_max_cells()); rows with more would-be cells get coarser ones.  One CTA per row, fp32.  theta, pulses and
+ * the schedule scalars are those of ddm_sim_f32 (no broadcast: ld_theta >= 5, ld_pulses >= P >= ceil(n_max /
+ * steps_per_pulse)).  A row whose theta is not finite, or whose 1 - lam dt is not positive, gives NaN.
+ *
+ * ddm_grid_law_f32: law_out_dev (N, 2, n_max): [r][c][k - 1] = P(choice c at step k) for k <= W, 0 after;
+ *   survive_out_dev (N,) = P(2), the mass still inside after W steps; cells_out_dev NULL or (N,) int32 = M.
+ * ddm_grid_loglik_f32: x_dev (N, 2) = [rt seconds, choice]; out_dev (N,) =
+ *   choice 0 / 1: log P(c, k) - log dt with k = rint((rt - t_nd) / dt), -inf unless 1 <= k <= W (a density in rt);
+ *   choice 2:     log P(2) (a probability mass).  Rows propagate only up to their observed step.
+ * ddm_grid_loglik_sum_f32: the potential's layout -- theta (C,5), x (T,2), pulses (T,>=P); row r = t * C + c is
+ *   (theta[c], x[t], pulses[t]); out[c] = sum over t = 0..T-1 in that order, in fp64, of the row values.
+ *   workspace_dev >= ddm_grid_loglik_sum_workspace_floats(T, C) floats; T * C < 2^31.
+ */
+int ddm_grid_max_cells(void);
+int ddm_grid_law_f32(const float *theta_dev, int64_t ld_theta, const float *pulses_dev, int64_t ld_pulses,
+                     int64_t N, int64_t P, int64_t n_max, int64_t steps_per_pulse, float dt, float t_max,
+                     float t_nd_hi, float noise_scale, float cells_per_sigma, float *law_out_dev,
+                     float *survive_out_dev, int32_t *cells_out_dev, void *stream);
+int ddm_grid_loglik_f32(const float *theta_dev, int64_t ld_theta, const float *x_dev, const float *pulses_dev,
+                        int64_t ld_pulses, int64_t N, int64_t P, int64_t n_max, int64_t steps_per_pulse, float dt,
+                        float t_max, float t_nd_hi, float noise_scale, float cells_per_sigma, float *out_dev,
+                        void *stream);
+size_t ddm_grid_loglik_sum_workspace_floats(int64_t T, int64_t C);
+int ddm_grid_loglik_sum_f32(const float *theta_dev, int64_t ld_theta, const float *x_dev, const float *pulses_dev,
+                            int64_t ld_pulses, int64_t T, int64_t C, int64_t P, int64_t n_max,
+                            int64_t steps_per_pulse, float dt, float t_max, float t_nd_hi, float noise_scale,
+                            float cells_per_sigma, float *out_dev, float *workspace_dev, void *stream);
+
 /* ------------------------------------------------------------ slice sampler --- */
 
 /*

@@ -47,6 +47,14 @@ _SIGNATURES = {
     "ddm_pcg64_advance": (ctypes.c_int, [_ptr, _ptr, _u64, _u64, _u64]),
     "ddm_slice_propose_f32": (ctypes.c_int, [_ptr, _ptr, _ptr, _ptr, _ptr]),
     "ddm_slice_update_f32": (ctypes.c_int, [_ptr, _ptr, _ptr, _ptr, _ptr]),
+    "ddm_grid_max_cells": (ctypes.c_int, []),
+    "ddm_grid_law_f32": (ctypes.c_int, [_ptr, _i64, _ptr, _i64, _i64, _i64, _i64, _i64, _f32, _f32, _f32, _f32, _f32,
+                                        _ptr, _ptr, _ptr, _ptr]),
+    "ddm_grid_loglik_f32": (ctypes.c_int, [_ptr, _i64, _ptr, _ptr, _i64, _i64, _i64, _i64, _i64, _f32, _f32, _f32, _f32,
+                                           _f32, _ptr, _ptr]),
+    "ddm_grid_loglik_sum_workspace_floats": (ctypes.c_size_t, [_i64, _i64]),
+    "ddm_grid_loglik_sum_f32": (ctypes.c_int, [_ptr, _i64, _ptr, _ptr, _i64, _i64, _i64, _i64, _i64, _i64, _f32, _f32,
+                                               _f32, _f32, _f32, _ptr, _ptr, _ptr]),
     "mnle_packed_floats": (ctypes.c_size_t, [_i32]),
     "mnle_create": (ctypes.c_int, [_ptr, ctypes.c_size_t, _i32, _ptr]),
     "mnle_destroy": (ctypes.c_int, [_ptr]),
