@@ -473,6 +473,24 @@ int ddm_grid_loglik_sum_f32(const float *theta_dev, int64_t ld_theta, const floa
                             int64_t steps_per_pulse, float dt, float t_max, float t_nd_hi, float noise_scale,
                             float cells_per_sigma, float *out_dev, float *workspace_dev, void *stream);
 
+/*
+ * ddm_grid_loglik_sum_batched_f32: D datasets in the potential's layout -- theta (D,C,5) (row d * C + c at
+ *   theta_dev + (d * C + c) * ld_theta), x (D,T,2), pulses (D,T,>=P) (row d * T + t at pulses_dev + (d * T + t) *
+ *   ld_pulses); out (D,C): out[d,c] = sum over t = 0..T-1 in that order, in fp64, of the ddm_grid_loglik_f32 value
+ *   of (theta[d,c], x[d,t], pulses[d,t]), bit for bit.  Each theta's weights of the steps without a kick are
+ *   tabulated once and applied to groups of its trials.  A theta that is not finite or has lam dt >= 0.5 gives NaN
+ *   (nothing is read on the host).  workspace_dev >= ddm_grid_loglik_sum_batched_workspace_floats(D, T, C,
+ *   cells_per_sigma) floats: the tables are built for a chunk of theta at a time (at most 1.75 GiB for any D * C),
+ *   plus 4 bytes per trial of all datasets (the trial order, D * T) and per (trial, theta) of a chunk; D * C < 2^31,
+ *   D * T < 2^31.
+ */
+size_t ddm_grid_loglik_sum_batched_workspace_floats(int64_t D, int64_t T, int64_t C, float cells_per_sigma);
+int ddm_grid_loglik_sum_batched_f32(const float *theta_dev, int64_t ld_theta, const float *x_dev,
+                                    const float *pulses_dev, int64_t ld_pulses, int64_t D, int64_t T, int64_t C,
+                                    int64_t P, int64_t n_max, int64_t steps_per_pulse, float dt, float t_max,
+                                    float t_nd_hi, float noise_scale, float cells_per_sigma, float *out_dev,
+                                    float *workspace_dev, void *stream);
+
 /* ------------------------------------------------------------ slice sampler --- */
 
 /*

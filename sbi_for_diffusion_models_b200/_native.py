@@ -55,6 +55,9 @@ _SIGNATURES = {
     "ddm_grid_loglik_sum_workspace_floats": (ctypes.c_size_t, [_i64, _i64]),
     "ddm_grid_loglik_sum_f32": (ctypes.c_int, [_ptr, _i64, _ptr, _ptr, _i64, _i64, _i64, _i64, _i64, _i64, _f32, _f32,
                                                _f32, _f32, _f32, _ptr, _ptr, _ptr]),
+    "ddm_grid_loglik_sum_batched_workspace_floats": (ctypes.c_size_t, [_i64, _i64, _i64, _f32]),
+    "ddm_grid_loglik_sum_batched_f32": (ctypes.c_int, [_ptr, _i64, _ptr, _ptr, _i64, _i64, _i64, _i64, _i64, _i64, _i64,
+                                                       _f32, _f32, _f32, _f32, _f32, _ptr, _ptr, _ptr]),
     "mnle_packed_floats": (ctypes.c_size_t, [_i32]),
     "mnle_create": (ctypes.c_int, [_ptr, ctypes.c_size_t, _i32, _ptr]),
     "mnle_destroy": (ctypes.c_int, [_ptr]),

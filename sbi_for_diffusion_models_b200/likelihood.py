@@ -11,7 +11,10 @@ error can be stated in nats per trial (``tools/mnle_vs_model.py``).
   k = round((rt - t_nd) / dt): a density in rt seconds, piecewise constant over each step, in the unit
   ``DeviceMNLE.log_prob`` uses.  For choice 2 it is log P(2), a probability MASS, which is not comparable with the
   estimator's density for choice 2.
-* ``GridLikelihood.loglik_sum``: the shape contract of ``DeviceMNLE.loglik_sum``.
+* ``GridLikelihood.loglik_sum`` / ``loglik_sum_batched``: the call shapes of ``DeviceMNLE.loglik_sum`` /
+  ``loglik_sum_batched``, so the MCMC drivers can sample the posterior under the model's own likelihood.  Each
+  theta's weights of the steps without a kick are tabulated once per call and shared by its trials; every value has
+  the bits of ``loglik_rows``.
 
 The discretisation, its truncation and its error are defined by ``oracle/ddm_grid_spec.py`` (float64) and
 DESIGN section 4b; the kernels are ``csrc/ddm_grid.cu``.  Schedule arguments default to the simulator's.
@@ -150,28 +153,48 @@ class GridLikelihood:
         self._device = device
 
     def loglik_sum(self, theta: torch.Tensor, x_o: torch.Tensor, pulses) -> torch.Tensor:
+        """The D = 1 case of ``loglik_sum_batched``, with the values of theta, x_o and pulses checked on the host."""
         sched = self.schedule
         theta = _check_theta(theta, sched, "GridLikelihood.loglik_sum")
-        C = theta.shape[0]
         x_o = x_o if isinstance(x_o, torch.Tensor) else torch.as_tensor(np.asarray(x_o))
         x_o = x_o.reshape(-1, 2)
         T = x_o.shape[0]
         x_o = _check_x(x_o, T, "GridLikelihood.loglik_sum")
         pl = _check_pulses(pulses, T, sched, "GridLikelihood.loglik_sum")
-        if T * C >= 2**31:
-            raise ValueError(f"GridLikelihood.loglik_sum: T * C must be < 2^31, got {T * C}")
+        return self.loglik_sum_batched(theta[None], x_o[None], pl[None])[0]
+
+    def loglik_sum_batched(self, theta: torch.Tensor, x_o: torch.Tensor, pulses: torch.Tensor) -> torch.Tensor:
+        """theta (D,C,5), x_o (D,T,2) = [rt seconds, choice], pulses (D,T,>=n_pulses) -> (D,C) fp32 with out[d,c] =
+        sum_t log p(x_o[d,t] | theta[d,c], pulses[d,t]), summed over t in order in fp64: the contract of
+        ``DeviceMNLE.loglik_sum_batched``.  Only shapes are checked and nothing is read back to the host, so a CUDA
+        graph can record the call; check the values of x_o and pulses once with the host checks of ``loglik_sum``.
+        A theta that is not finite or has lam * dt >= 0.5 gives NaN."""
+        sched = self.schedule
+        if theta.ndim != 3 or theta.shape[2] != 5:
+            raise ValueError(f"GridLikelihood.loglik_sum_batched: theta must be (D,C,5), got {tuple(theta.shape)}")
+        D, C = theta.shape[0], theta.shape[1]
+        if x_o.ndim != 3 or x_o.shape[0] != D or x_o.shape[2] != 2:
+            raise ValueError(f"GridLikelihood.loglik_sum_batched: x_o must be (D,T,2) with D={D}, got {tuple(x_o.shape)}")
+        T = x_o.shape[1]
+        if pulses.ndim != 3 or pulses.shape[0] != D or pulses.shape[1] != T or pulses.shape[2] < sched.n_pulses:
+            raise ValueError(f"GridLikelihood.loglik_sum_batched: pulses must be (D,T,>={sched.n_pulses}) with D={D}, "
+                             f"T={T}, got {tuple(pulses.shape)}")
+        if D * C >= 2**31 or D * T >= 2**31:
+            raise ValueError(f"GridLikelihood.loglik_sum_batched: D * C and D * T must be < 2^31, got {D * C}, {D * T}")
         L = _native.lib()
         dev = compute_device(self._device if self._device is not None else (theta.device if theta.is_cuda else None))
         with torch.cuda.device(dev):
-            th = _as_f32_rows(theta, dev).contiguous()
-            xr = _as_f32_rows(x_o, dev).contiguous()
-            s = _as_f32_rows(pl, dev).contiguous()
-            out = torch.empty((C,), dtype=torch.float32, device=dev)
-            ws = torch.empty((max(L.ddm_grid_loglik_sum_workspace_floats(T, C), 1),), dtype=torch.float32, device=dev)
-            rc = L.ddm_grid_loglik_sum_f32(th.data_ptr() if C else None, 5, xr.data_ptr() if T else None,
-                                           s.data_ptr() if T else None, s.shape[1], T, C, s.shape[1], sched.n_max,
-                                           sched.steps_per_pulse, sched.dt, sched.t_max, sched.t_nd_hi,
-                                           sched.noise_scale, self.cells_per_sigma, out.data_ptr() if C else None,
-                                           ws.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
-            _native.check(rc, "ddm_grid_loglik_sum_f32")
+            th = theta.to(device=dev, dtype=torch.float32).contiguous()
+            xr = x_o.to(device=dev, dtype=torch.float32).contiguous()
+            s = pulses.to(device=dev, dtype=torch.float32).contiguous()
+            out = torch.empty((D, C), dtype=torch.float32, device=dev)
+            n_ws = L.ddm_grid_loglik_sum_batched_workspace_floats(D, T, C, self.cells_per_sigma)
+            ws = torch.empty((max(n_ws, 1),), dtype=torch.float32, device=dev)
+            rc = L.ddm_grid_loglik_sum_batched_f32(th.data_ptr() if D * C else None, 5, xr.data_ptr() if D * T else None,
+                                                   s.data_ptr() if D * T else None, s.shape[2], D, T, C, s.shape[2],
+                                                   sched.n_max, sched.steps_per_pulse, sched.dt, sched.t_max,
+                                                   sched.t_nd_hi, sched.noise_scale, self.cells_per_sigma,
+                                                   out.data_ptr() if D * C else None, ws.data_ptr(),
+                                                   torch.cuda.current_stream(dev).cuda_stream)
+            _native.check(rc, "ddm_grid_loglik_sum_batched_f32")
         return out.to(theta.device)

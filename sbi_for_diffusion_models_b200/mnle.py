@@ -20,24 +20,28 @@ from typing import Optional, Sequence
 import numpy as np
 import torch
 
+from .likelihood import GridLikelihood, _check_pulses, _check_x
 from .potentials import as_device_estimator, prior_log_prob
 from .samplers import GraphedLogProb, PhiloxUniforms, VectorizedSliceSampler
 from .sbc import compute_ranks, draw_sbc_datasets, simulate_sbc_sessions
 from .sharding import _world, all_gather_rows, gather_sbc, shard_bounds
-from .simulator import compute_device
+from .simulator import Schedule, compute_device
 
 MIN_VECTOR_CHAINS = 128   # one row tile of the potential kernel
 
 
-def _init_from_prior(prior_theta, log_prob_fn, n: int, device, max_tries: int = 20) -> torch.Tensor:
+def _init_from_prior(prior_theta, log_prob_fn, n: int, device, max_tries: int = 1000) -> torch.Tensor:
     """``init_strategy="proposal"`` (reference mnle.py:85): prior draws, redrawn where the
-    posterior potential is not finite."""
+    posterior potential is not finite.  Only the redrawn rows are evaluated again: under the grid likelihood every
+    draw whose t_nd comes after the session's first rt has zero likelihood, and that can be most of the prior."""
     x = prior_theta.sample((n,)).to(device=device, dtype=torch.float32)
+    bad = ~torch.isfinite(log_prob_fn(x))
     for _ in range(max_tries):
-        bad = ~torch.isfinite(log_prob_fn(x))
         if not bool(bad.any()):
             return x
-        x[bad] = prior_theta.sample((int(bad.sum()),)).to(device=device, dtype=torch.float32)
+        rows = bad.nonzero()[:, 0]
+        x[rows] = prior_theta.sample((rows.numel(),)).to(device=device, dtype=torch.float32)
+        bad[rows] = ~torch.isfinite(log_prob_fn(x[rows]))
     raise RuntimeError("could not find starting points with finite posterior potential")
 
 
@@ -61,13 +65,25 @@ def run_inference_mcmc(cfg, prior_theta, density_estimator, x_o, pulses_o, *, nu
         x = x[:, 0, :]
     pulses = pulses_o.to(device=dev, dtype=torch.float32)
     assert pulses.shape[0] == x.shape[0], f"local_theta must have shape (num_trials, P). Got {tuple(pulses.shape)}"
-    fn = _BatchedPotential(as_device_estimator(density_estimator), prior_theta, x[None], pulses[None], float(cfg.TEMPERATURE))
+    est = _potential_estimator(density_estimator, x, pulses, "run_inference_mcmc")
+    fn = _BatchedPotential(est, prior_theta, x[None], pulses[None], float(cfg.TEMPERATURE))
     init = _init_from_prior(prior_theta, fn, chains, dev)
     sampler = VectorizedSliceSampler(GraphedLogProb(fn, init), init, generator=generator)
     want = int(cfg.POSTERIOR_SAMPLES)
     per_chain = -(-want // chains)
     draws = sampler.run(per_chain, warmup=int(cfg.WARMUP_STEPS), thin=1)          # (per_chain, chains, 5)
     return draws.reshape(-1, draws.shape[-1])[:want].detach().cpu()
+
+
+def _potential_estimator(density_estimator, x, pulses, what: str):
+    """The estimator a potential drives: a ``GridLikelihood`` as it is (the model's own likelihood; the values of x
+    and pulses are checked here, once), anything else through ``as_device_estimator``."""
+    if isinstance(density_estimator, GridLikelihood):
+        sched = density_estimator.schedule
+        _check_x(x.reshape(-1, 2), x.numel() // 2, what)
+        _check_pulses(pulses.reshape(-1, pulses.shape[-1]), x.numel() // 2, sched, what)
+        return density_estimator
+    return as_device_estimator(density_estimator)
 
 
 class _BatchedPotential:
@@ -126,6 +142,8 @@ def sbc_shard(cfg, prior_theta, estimator, thetas_true: torch.Tensor, ds_seeds, 
     if bool(cfg.LOG_RT_MANUALLY):
         x = x.clone()
         x[..., 0] = torch.log(x[..., 0].clamp_min(1e-6))
+    if isinstance(estimator, GridLikelihood):
+        _potential_estimator(estimator, x, pulses, "sbc_shard")
     potential = _BatchedPotential(estimator, prior_theta, x, pulses, float(cfg.TEMPERATURE))
     init = init_all[lo * C:hi * C].to(device=dev, dtype=torch.float32)
     samples = _sample_groups(cfg, potential, init, D, lo, S, seed, "dataset")
@@ -146,14 +164,24 @@ def run_sbc(cfg, *, prior_theta, density_estimator, device: str = "cpu", num_dat
     "all_samples": list of N CPU tensors (S,5)} on every rank, identical for any number of ranks.
     ``device`` is accepted for signature compatibility; the work runs on this rank's GPU."""
     dev = compute_device(None)
+    if isinstance(density_estimator, GridLikelihood):
+        # the sessions are simulated with the simulator's schedule at cfg.MU_SENSORY and rt in seconds
+        if density_estimator.schedule != Schedule.from_constants(float(cfg.MU_SENSORY)):
+            raise ValueError("run_sbc: the grid likelihood's schedule is not the one the sessions are simulated with "
+                             f"(Schedule.from_constants({float(cfg.MU_SENSORY)}))")
+        if bool(cfg.LOG_RT_MANUALLY):
+            raise ValueError("run_sbc: the grid likelihood needs rt in seconds, but cfg.LOG_RT_MANUALLY is set")
+        estimator = density_estimator
+    else:
+        estimator = as_device_estimator(density_estimator)
     rank, world = _world(group)
     N = int(num_datasets)
     S = int(posterior_samples_per_dataset) if posterior_samples_per_dataset is not None else int(cfg.POSTERIOR_SAMPLES)
     thetas_true, ds_seeds = draw_sbc_datasets(prior_theta, N, seed)                       # reference order
     init_all = prior_theta.sample((N * int(chains_per_dataset),)).to(torch.float32)       # same on every rank
     lo, hi = shard_bounds(N, rank, world)
-    ranks_local, samples_local = sbc_shard(cfg, prior_theta, as_device_estimator(density_estimator), thetas_true, ds_seeds,
-                                           init_all, lo, hi, S, seed, dev)
+    ranks_local, samples_local = sbc_shard(cfg, prior_theta, estimator, thetas_true, ds_seeds, init_all, lo, hi, S, seed,
+                                           dev)
     thetas_all, ranks_all = gather_sbc(thetas_true[lo:hi].to(dev), ranks_local.to(dev), N, group)
     samples_all = all_gather_rows(samples_local.to(dev), N, group).cpu()
     out = {"thetas_true": thetas_all.cpu().numpy(), "ranks": ranks_all.cpu().numpy(),
@@ -214,6 +242,9 @@ def run_inference_sessions(cfg, prior_theta, density_estimator, sessions, *, num
     is left alone), the sampler's uniforms are keyed by ``seed`` and the global chain number.  Under torchrun the
     sessions are split over the ranks (``shard_bounds``) and the draws all-gathered: every rank returns the full
     list, identical for any world size."""
+    if isinstance(density_estimator, GridLikelihood):
+        raise TypeError("run_inference_sessions: the grid likelihood has no ragged-session potential; sample each "
+                        "session with run_inference_mcmc")
     sessions = list(sessions)
     n = len(sessions)
     if n == 0:
